@@ -2,6 +2,7 @@
 """Benchmark of the ModalTune-GigaPath fine-tuning hot path (BASELINE.json: slides/s fwd+bwd at 10k tiles).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--tiles L] [--mode bf16|fp32]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one slide through the reference's training step: 3 task passes forward, the KL-distillation loss, one backward
@@ -19,8 +20,9 @@ rank processes its own slides (weak scaling, no data-path collective).  Prints O
   tensor peak of MEASURED_PEAKS.json.
 * ``cpu_baseline`` / ``--impl reference``: the oracle port of the reference's CPU arithmetic (the reference is pure
   Python and has no CPU attention of its own) on the host cores: ``cpu_baseline`` = SURVEY.md 8(d)'s C1 protocol (COMPLETE
-  oracle training steps at 1 024 tiles, 1 warm-up + 3 timed, median); ``--impl reference`` = complete oracle training
-  steps at the bench tile count, as many as fit the CPU budget, reporting the true ``steps`` it ran (never a scaled figure).
+  oracle training steps at 1 024 tiles, 1 warm-up + 3 timed, median); ``--impl reference`` = ``--steps`` complete oracle
+  training steps at the bench tile count (fewer only under an explicit ``--cpu-budget``), reporting the true ``steps``
+  it ran (never a scaled figure).
 """
 import argparse
 import json
@@ -47,13 +49,23 @@ def parse():
     ap.add_argument("--mode", default="bf16", choices=["bf16", "fp32"])
     ap.add_argument("--attn", default="auto", choices=["auto", "simt", "sm100"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--cpu-budget", type=float, default=200.0, help="seconds of oracle steps the reference arm may time")
+    ap.add_argument("--cpu-budget", type=float, default=None,
+                    help="cap on the seconds of oracle steps the reference arm times (default: no cap, all --steps run)")
     ap.add_argument("--no-extras", action="store_true", help="skip the comparator / 32k / train-mode sub-records")
     ap.add_argument("--no-graph", action="store_true", help="issue every step eagerly instead of replaying a CUDA graph")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (loss, logits, gradients) to DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU step (--impl ours)")
+    return args
 
 
 UNIT = "slides/s"
+# gradient elements --dump-outputs writes: a fixed seeded sample, 16 MB of the 135 MB fp32 gradient of the full model
+DUMP_GRAD_SAMPLE = 1 << 22
 # DRAM bytes of ONE launch of the default backward attention kernel at 10 001 tokens, from the committed `ncu --set full`
 # capture (profiles/r2_ncu_attention.txt)
 NCU_TRAFFIC_BWD = 243.571712e6 + 96.210176e6
@@ -78,6 +90,23 @@ def workload_config(args, world):
         "slides_per_step_per_gpu": 1, "parallelism": f"slide-sharded dp{world}",
         "l2": "working set per step (several GB of saved activations) exceeds the 126 MB L2; no explicit flush",
     }
+
+
+def dump_outputs(out_dir: str, loss, logits, params) -> None:
+    """``--dump-outputs``: what a caller of the step receives, as .npy files that two builds can be compared on.
+    ``loss`` (float32 scalar), ``logits`` (float32 [3, 256]), ``grad_norms`` (float64, the L2 norm of every trainable
+    parameter's gradient in ``named_parameters`` order) and ``grad_sample`` (float32: the flat gradient vector, in the same
+    order, at ``DUMP_GRAD_SAMPLE`` positions drawn with a fixed seed; all of it when it is shorter)."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    grads = [(p.grad if p.grad is not None else torch.zeros_like(p)).detach().float().reshape(-1) for p in params]
+    flat = torch.cat(grads)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_GRAD_SAMPLE].sort().values
+    arrays = {"loss": loss.detach().float().reshape(()), "logits": logits.detach().float(),
+              "grad_norms": torch.stack([g.double().norm() for g in grads]), "grad_sample": flat[idx.to(flat.device)]}
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.cpu().numpy())
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -158,19 +187,21 @@ def cpu_baseline(tiles: int):
 
 
 def run_reference(args):
-    """``--impl reference``: complete oracle training steps at the bench tile count on the host cores.  A step takes
-    about a minute at 10k tiles, so the run does as many of the requested steps as fit ``--cpu-budget`` seconds (at
-    least one) and reports the TRUE ``steps`` / ``warmup`` it ran and the measured mean, never a scaled figure."""
+    """``--impl reference``: ``--steps`` complete oracle training steps at the bench tile count on the host cores, after
+    one warm-up step when ``--warmup`` > 0.  A step takes about a minute at 10k tiles: ``--cpu-budget S`` caps the run
+    at as many steps as fit S seconds (at least one).  Either way the TRUE ``steps`` / ``warmup`` it ran and the measured
+    mean are reported, never a scaled figure."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
+    budget = float("inf") if args.cpu_budget is None else args.cpu_budget
     step = CpuStep(args.tiles)
     t_first = step(0)
-    warm = 1 if (args.warmup > 0 and 3.0 * t_first < args.cpu_budget) else 0
+    warm = 1 if (args.warmup > 0 and 3.0 * t_first < budget) else 0
     ts = [] if warm else [t_first]
     spent = t_first
     i = 1
-    while len(ts) < args.steps and (not ts or spent + ts[-1] < args.cpu_budget):
+    while len(ts) < args.steps and (not ts or spent + ts[-1] < budget):
         ts.append(step(i))
         spent += ts[-1]
         i += 1
@@ -186,7 +217,8 @@ def run_reference(args):
                                    f"pathways{', every encoder layer recomputed in the backward (activation checkpointing)' if step.checkpoint else ''}) "
                                    f"at {args.tiles} tiles, {torch.get_num_threads()} threads, "
                                    f"{'1 full warm-up step' if warm else 'warm-up = one untimed 256-tile step'}; steps in seconds: "
-                                   f"{[round(x, 1) for x in ts]}; stopped at the {args.cpu_budget:.0f} s budget; the "
+                                   f"{[round(x, 1) for x in ts]}; {len(ts)} of {args.steps} requested steps"
+                                   f"{'' if args.cpu_budget is None else f' under the {args.cpu_budget:.0f} s budget'}; the "
                                    f"reference is pure Python with no CPU attention kernel of its own "
                                    f"(flash_attn_func is None on CPU), so the arm is the oracle port pinned by tests/golden"},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
@@ -473,8 +505,16 @@ def main():
     if rank == 0:
         clocks.start()
     launches0 = ops.launch_count
-    ms = timed(lambda i: step(resident[i % n_slides]), args.steps)
+    last = [None]
+
+    def resident_step(i):
+        last[0] = step(resident[i % n_slides])
+
+    ms = timed(resident_step, args.steps)
     value = world * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        # before the e2e region below replays the graph again and overwrites its outputs
+        dump_outputs(args.dump_outputs, *last[0], [p for p in model.parameters() if p.requires_grad])
 
     # ---- end to end: pinned host -> device, step, loss/logits back to the host ---------------------------------------
     out = {}

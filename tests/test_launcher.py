@@ -34,7 +34,7 @@ def _reference_or_skip():
         staged = os.path.join(ROOT, "oracle", "_ref", "reference")   # test infrastructure: staged by build()
         return launcher.find_reference(staged if os.path.isdir(staged) and not os.path.isdir("/root/reference") else None)
     except FileNotFoundError:
-        pytest.skip("no reference checkout (build container: /root/reference; GPU box: oracle/_ref/reference)")
+        pytest.skip("needs a checkout of the original ModalTune project: set MODALTUNE_REFERENCE to it")
 
 
 def _losses(text):

@@ -24,7 +24,8 @@ from modaltune_b200 import config, synthetic
 from tests import cpu_kernels, helpers
 from tests.golden import ref_shims
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(ref_shims.REFERENCE_ROOT), reason="needs the reference tree")
+pytestmark = pytest.mark.skipif(not os.path.isdir(ref_shims.REFERENCE_ROOT),
+                                reason="needs a checkout of the original ModalTune project: set MODALTUNE_REFERENCE to it")
 
 L_TILES, N_CASES = 200, 2
 
