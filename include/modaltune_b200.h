@@ -82,7 +82,8 @@ int mt_layernorm_fwd(const void* x, int x_dtype, const float* gamma, const float
                      float eps, void* stream);
 /* bwd: dx = LN'(dy) [+ residual];  optional dgamma/dbeta [cols] f32 (accumulated with atomics into zeroed buffers);
  * dx_bf16 (or NULL): a second copy of dx rounded to bf16, written in the same pass for the GEMM that consumes the
- * gradient next (saves a separate cast pass over [rows, cols]). */
+ * gradient next (saves a separate cast pass over [rows, cols]).  `residual` may be `dx` itself (an in-place add, same
+ * dtype): every element is read once, by the thread that then writes it. */
 int mt_layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma, const float* mean,
                      const float* rstd, const void* residual, int res_dtype, void* dx, int dx_dtype, void* dx_bf16,
                      float* dgamma, float* dbeta, int64_t rows, int64_t cols, void* stream);
