@@ -87,6 +87,15 @@ int mt_layernorm_fwd(const void* x, int x_dtype, const float* gamma, const float
 int mt_layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma, const float* mean,
                      const float* rstd, const void* residual, int res_dtype, void* dx, int dx_dtype, void* dx_bf16,
                      float* dgamma, float* dbeta, int64_t rows, int64_t cols, void* stream);
+/* deterministic mt_layernorm_bwd: dgamma / dbeta are not accumulated with atomics but written (no zeroing needed): every
+ * block stores its column partials to `workspace` and a second pass adds them in block order, so the same inputs give
+ * the same bits in every run.  workspace_floats >= mt_colreduce_workspace_floats(cols) when dgamma is not NULL. */
+int mt_layernorm_bwd_ws(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma, const float* mean,
+                        const float* rstd, const void* residual, int res_dtype, void* dx, int dx_dtype, void* dx_bf16,
+                        float* dgamma, float* dbeta, int64_t rows, int64_t cols, float* workspace,
+                        int64_t workspace_floats, void* stream);
+/* workspace of the deterministic column reductions (mt_layernorm_bwd_ws, mt_gated_residual_bwd_ws, mt_colsum_ws) */
+int64_t mt_colreduce_workspace_floats(int64_t cols);
 
 /* mt_layernorm_bwd (f32 tensors, cols = 768, residual and bf16 twin required) of the pre-attention LayerNorm of layer
  * l + 1 that ALSO does mt_ffn_bwd_prep for layer l: its dx IS layer l's dy and its x IS layer l's output y, so the row means
@@ -186,7 +195,8 @@ int mt_ffn_bwd_prep(const float* dy, const float* y, const float* x1, const floa
  * impl: 0 = SIMT fp32 math (any dtype; also the on-device cross-check of the tensor-core kernels), >= 1 = tcgen05 / TMA /
  * TMEM kernels (bf16 only): 1 = one CTA per work item, 2 (backward only) = persistent CTAs that pull work items from a
  * device counter (identical arithmetic; hands over between items without draining its pipeline; the default backward),
- * 3 (forward only) = one CTA per work item with 48-key score tiles, four CTAs per SM (the default forward).  A shared-memory window that is not 1024-byte aligned (never expected) makes the tcgen05
+ * 3 (forward only) = one CTA per work item with 48-key score tiles, four CTAs per SM (the default forward),
+ * 4 (backward only) = the deterministic backward (MT_DILATED_BWD_DETERMINISTIC below).  A shared-memory window that is not 1024-byte aligned (never expected) makes the tcgen05
  * kernels trap: the failure surfaces as a CUDA error on the stream, never as silently unwritten outputs. */
 int mt_dilated_attn_fwd(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc, int dtype,
                         void* o_br, float* lse_br, int impl, void* stream);
@@ -211,6 +221,12 @@ int mt_dilated_merge_ln_bwd(const mt_dilated_geometry* geom, const void* dy, int
 int mt_dilated_attn_bwd(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
                         const void* dattn, const float* lse, const float* delta_br, int dtype, float* dqkv_f32,
                         int impl, void* stream);
+/* impl 4 (bf16, tcgen05): the DETERMINISTIC backward -- the same inputs give bitwise the same dqkv in every run.  Every
+ * element of dqkv receives at most one non-zero addition per branch, and the branches are added in a fixed order: the
+ * branches run one after another on the stream (b = 0 .. n_branches - 1), each as a query-major dQ kernel (one CTA per
+ * query tile streams the key tiles of its segment, dQ leaves once) and a key-major dK / dV kernel (impl 1 without
+ * its dQ part).  About 3.5x the forward's tensor work instead of 2.5x. */
+#define MT_DILATED_BWD_DETERMINISTIC 4
 
 /* ---- A7/A8: Injector / Extractor cross-attention core (12 heads x 16) ---------------------------------------------
  * replaces: the softmax(QK^T/4)V inside nn.MultiheadAttention called from CrossAttentionLayer.forward_pre
@@ -229,6 +245,14 @@ int mt_cross_attn_bwd(const void* q, int64_t ldq, const void* k, const void* v, 
                       float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads, int head_dim,
                       int impl, void* stream);
 int64_t mt_cross_attn_workspace_floats(int64_t lq, int64_t lk, int heads, int head_dim, int dtype, int impl);
+/* deterministic mt_cross_attn_bwd (impl 1, f32 tensors): a loop that is split over CTAs stores its partials to
+ * `workspace` ([splits][rows][heads * head_dim]) instead of adding them with atomics, and a second pass sums the splits in
+ * index order; unsplit loops store as before.  workspace_floats >= mt_cross_attn_bwd_workspace_floats(...) (may be 0). */
+int mt_cross_attn_bwd_ws(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* o,
+                         const void* d_o, int64_t ldo, const float* lse, int dtype, float* dq_f32, int64_t lddq,
+                         float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads, int head_dim,
+                         float* workspace, int64_t workspace_floats, int impl, void* stream);
+int64_t mt_cross_attn_bwd_workspace_floats(int64_t lq, int64_t lk, int heads, int head_dim, int dtype, int impl);
 
 /* ---- small fused element-wise pieces ------------------------------------------------------------------------------
  * y[r, c] = a[r, c] + gate[c] * (a[r, c] + b[r, c])      Injector tail `query + gamma * attn` (adapter_modules.py:362)
@@ -240,6 +264,11 @@ int mt_gated_residual(const float* a, const void* b, int b_dtype, const float* g
  * gets the bias gradient of the projection that produced b (gate * dysum) without a reduction pass over db. */
 int mt_gated_residual_bwd(const float* dy, const float* a, const void* b, int b_dtype, const float* gate, float* da,
                           void* db, int db_dtype, float* dgate, float* dysum, int64_t rows, int64_t cols, void* stream);
+/* deterministic mt_gated_residual_bwd: dgate / dysum from block partials in `workspace` added in block order
+ * (workspace_floats >= mt_colreduce_workspace_floats(cols)). */
+int mt_gated_residual_bwd_ws(const float* dy, const float* a, const void* b, int b_dtype, const float* gate, float* da,
+                             void* db, int db_dtype, float* dgate, float* dysum, int64_t rows, int64_t cols,
+                             float* workspace, int64_t workspace_floats, void* stream);
 /* y = x + D(a + bias): residual add after fc2 (torchscale/architecture/encoder.py:169-175), bias [cols] f32 or NULL,
  * D = dropout + DropPath of the branch (drop NULL = identity). */
 int mt_residual_bias_add(const float* x, const void* a, int a_dtype, const float* bias, float* y, int64_t rows,
@@ -248,6 +277,9 @@ int mt_cast(const void* src, int src_dtype, void* dst, int dst_dtype, int64_t n,
 /* out[c] = sum_r x[r, c]: the bias gradient `dy.sum(0)` of the adapter's projections (autograd of nn.Linear in
  * models/vitadapter/adapter_modules.py:210-234); x [rows, cols] f32 with row stride ld, cols % 4 == 0, <= 4096. */
 int mt_colsum(const float* x, int64_t ld, float* out, int64_t rows, int64_t cols, void* stream);
+/* deterministic mt_colsum: block partials in `workspace` added in block order (>= mt_colreduce_workspace_floats(cols)) */
+int mt_colsum_ws(const float* x, int64_t ld, float* out, int64_t rows, int64_t cols, float* workspace,
+                 int64_t workspace_floats, void* stream);
 /* backward of D: dst[i] = src[i] * keep_mask(i) / (1 - p) * path_scale, converted to dst_dtype (the gradient that
  * enters the dX GEMM of the branch).  drop must not be NULL. */
 int mt_dropout_bwd_cast(const void* src, int src_dtype, void* dst, int dst_dtype, int64_t n, const mt_dropout* drop,

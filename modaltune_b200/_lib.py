@@ -61,6 +61,9 @@ SIGNATURES = {
     "mt_embed_assemble": (c_int, [_P, c_int, _P, _P, _P, _P, _P, _I64, _I64, _I64, c_float, _P]),
     "mt_layernorm_fwd": (c_int, [_P, c_int, _P, _P, _P, c_int, _I64, _P, c_int, _P, _P, _I64, _I64, c_float, _P]),
     "mt_layernorm_bwd": (c_int, [_P, c_int, _P, c_int, _P, _P, _P, _P, c_int, _P, c_int, _P, _P, _P, _I64, _I64, _P]),
+    "mt_layernorm_bwd_ws": (c_int, [_P, c_int, _P, c_int, _P, _P, _P, _P, c_int, _P, c_int, _P, _P, _P, _I64, _I64, _P, _I64,
+                                    _P]),
+    "mt_colreduce_workspace_floats": (_I64, [_I64]),
     "mt_layernorm_bwd_ffn_prep": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
     "mt_add_layernorm_fwd": (c_int, [_P, _P, c_int, _P, _P, _P, _P, _P, c_int, _P, _P, _I64, _I64, c_float, _D, _P]),
     "mt_gelu_ln_fwd": (c_int, [_P, c_int, _P, _P, _P, _P, c_int, _P, _P, _I64, _I64, c_float, _P]),
@@ -75,12 +78,17 @@ SIGNATURES = {
     "mt_cross_attn_bwd": (c_int, [_P, _I64, _P, _P, _I64, _P, _P, _I64, _P, c_int, _P, _I64, _P, _P, _I64, _I64, _I64, c_int,
                                   c_int, c_int, _P]),
     "mt_cross_attn_workspace_floats": (_I64, [_I64, _I64, c_int, c_int, c_int, c_int]),
+    "mt_cross_attn_bwd_ws": (c_int, [_P, _I64, _P, _P, _I64, _P, _P, _I64, _P, c_int, _P, _I64, _P, _P, _I64, _I64, _I64,
+                                     c_int, c_int, _P, _I64, c_int, _P]),
+    "mt_cross_attn_bwd_workspace_floats": (_I64, [_I64, _I64, c_int, c_int, c_int, c_int]),
     "mt_gated_residual": (c_int, [_P, _P, c_int, _P, _P, _I64, _I64, _P]),
     "mt_gated_residual_bwd": (c_int, [_P, _P, _P, c_int, _P, _P, _P, c_int, _P, _P, _I64, _I64, _P]),
+    "mt_gated_residual_bwd_ws": (c_int, [_P, _P, _P, c_int, _P, _P, _P, c_int, _P, _P, _I64, _I64, _P, _I64, _P]),
     "mt_residual_bias_add": (c_int, [_P, _P, c_int, _P, _P, _I64, _I64, _D, _P]),
     "mt_dropout_bwd_cast": (c_int, [_P, c_int, _P, c_int, _I64, _D, _P]),
     "mt_cast": (c_int, [_P, c_int, _P, c_int, _I64, _P]),
     "mt_colsum": (c_int, [_P, _I64, _P, _I64, _I64, _P]),
+    "mt_colsum_ws": (c_int, [_P, _I64, _P, _I64, _I64, _P, _I64, _P]),
 }
 
 _lib = None

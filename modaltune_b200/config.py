@@ -7,11 +7,16 @@
 ``attn_impl``
     ``"auto"`` -- tcgen05/TMA dilated-attention kernels in bf16 mode, SIMT kernels in fp32 mode;
     ``"simt"`` -- force the SIMT kernels (any mode);  ``"sm100"`` -- force the tcgen05 kernels (bf16 only).
+``deterministic``
+    bitwise-reproducible backward: every gradient reduction of the project's kernels runs in a fixed order, so the same
+    seeded step gives the same loss, logits, gradients and optimizer updates in every run.  On with
+    ``MODALTUNE_B200_DETERMINISTIC=1``, ``using(deterministic=True)`` or ``torch.use_deterministic_algorithms(True)``.
 """
 from __future__ import annotations
 
 import contextlib
 import os
+import warnings
 
 import torch
 
@@ -34,6 +39,7 @@ _state = {
     "injector_fused": os.environ.get("MODALTUNE_B200_INJECTOR_FUSED", "1") != "0",     # ops.InjectorFn
     "split_param_grads": os.environ.get("MODALTUNE_B200_SPLIT_GRADS", "1") != "0",     # per-pass leaf aliases
     "cross_tc": os.environ.get("MODALTUNE_B200_CROSS_TC", "1") != "0",                 # TF32 tensor-core cross-attention
+    "deterministic": os.environ.get("MODALTUNE_B200_DETERMINISTIC", "0") not in ("", "0"),
 }
 
 
@@ -105,10 +111,38 @@ def compute_dtype() -> torch.dtype:
 AUTO_IMPL = {"fwd": 3, "bwd": 2}
 
 
+# the deterministic backward of the dilated attention (mt_dilated_attn_bwd impl 4, include/modaltune_b200.h)
+DETERMINISTIC_BWD_IMPL = 4
+
+
+def deterministic() -> bool:
+    """Is deterministic mode on: the switch (``MODALTUNE_B200_DETERMINISTIC=1`` / ``set_deterministic``) or torch's
+    ``torch.use_deterministic_algorithms(True)``."""
+    return _state["deterministic"] or torch.are_deterministic_algorithms_enabled()
+
+
+def set_deterministic(on: bool) -> None:
+    _state["deterministic"] = bool(on)
+
+
+def check_deterministic(what: str) -> None:
+    """``what`` has no deterministic variant: in deterministic mode raise, as torch does for its own ops (or warn when
+    torch's flag is set with ``warn_only=True``)."""
+    if not deterministic():
+        return
+    msg = (f"{what} adds gradients in arbitrary order and has no deterministic variant; deterministic mode needs bf16 "
+           "mode with the tcgen05 attention kernels (attn_impl auto / sm100) and the tensor-core cross-attention")
+    if not _state["deterministic"] and torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(msg)
+        return
+    raise RuntimeError(msg)
+
+
 def attn_impl(direction: str = "fwd") -> int:
     """The ``impl`` argument of mt_dilated_attn_{fwd,bwd}: 0 = SIMT, 1 / 2 = tcgen05 (forward: O accumulated in TMEM
     with a lazily raised row maximum; backward: transposed formulation, per-query statistics folded into the MMAs, TMA
-    reduce-adds for dQ / dK / dV), 2 = persistent CTAs."""
+    reduce-adds for dQ / dK / dV), 2 = persistent CTAs.  In deterministic mode ``ops.dilated_attn_bwd`` runs the
+    tcgen05 backward as impl 4 (``DETERMINISTIC_BWD_IMPL``)."""
     impl = _state["attn_impl"]
     if impl == "simt" or _state["mode"] == "fp32":
         if impl == "sm100":
@@ -118,7 +152,8 @@ def attn_impl(direction: str = "fwd") -> int:
 
 
 @contextlib.contextmanager
-def using(mode: str | None = None, attn_impl: str | None = None, gemm: str | None = None):
+def using(mode: str | None = None, attn_impl: str | None = None, gemm: str | None = None,
+          deterministic: bool | None = None):
     old = dict(_state)
     try:
         if mode is not None:
@@ -127,6 +162,8 @@ def using(mode: str | None = None, attn_impl: str | None = None, gemm: str | Non
             set_attn_impl(attn_impl)
         if gemm is not None:
             set_gemm_impl(gemm)
+        if deterministic is not None:
+            set_deterministic(deterministic)
         yield
     finally:
         _state.update(old)

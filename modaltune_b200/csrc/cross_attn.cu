@@ -563,7 +563,7 @@ __device__ __forceinline__ void cross_bwd_dq_tc(BwdSmem& sm, int bx, int h, int 
                                                 const float* __restrict__ v, const float* __restrict__ o,
                                                 const float* __restrict__ d_o, const float* __restrict__ lse,
                                                 float* __restrict__ dq, int64_t lq, int64_t lk, int heads,
-                                                int64_t keys_per_split, const Strides& sd) {
+                                                int64_t keys_per_split, const Strides& sd, float* __restrict__ part) {
   uint32_t* Ks = sm.a;
   uint32_t* Vs = sm.b;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
@@ -621,6 +621,8 @@ __device__ __forceinline__ void cross_bwd_dq_tc(BwdSmem& sm, int bx, int h, int 
       float2* dst = reinterpret_cast<float2*>(dq + r * sd.dq + h * HD + 8 * d + 2 * t);
       const float2 val = make_float2(acc[d][2 * half] * 0.25f, acc[d][2 * half + 1] * 0.25f);
       if (nsplit == 1) *dst = val;
+      else if (part != nullptr)   // deterministic: [split][lq][heads * HD], summed in split order by cross_split_sum_kernel
+        *reinterpret_cast<float2*>(part + ((int64_t)split * lq + r) * heads * HD + h * HD + 8 * d + 2 * t) = val;
       else atomicAdd(dst, val);
     }
   }
@@ -633,7 +635,8 @@ __device__ __forceinline__ void cross_bwd_dkv_tc(BwdSmem& sm, int bx, int h, int
                                                  const float* __restrict__ v, const float* __restrict__ o,
                                                  const float* __restrict__ d_o, const float* __restrict__ lse,
                                                  float* __restrict__ dk, float* __restrict__ dv, int64_t lq,
-                                                 int64_t lk, int heads, int64_t q_per_split, const Strides& sd) {
+                                                 int64_t lk, int heads, int64_t q_per_split, const Strides& sd,
+                                                 float* __restrict__ part) {
   uint32_t* Qs = sm.a;
   uint32_t* Gs = sm.b;
   float* Ls = sm.ls;
@@ -717,6 +720,10 @@ __device__ __forceinline__ void cross_bwd_dkv_tc(BwdSmem& sm, int bx, int h, int
       if (nsplit == 1) {
         *dstk = vk;
         *dstv = vv;
+      } else if (part != nullptr) {   // deterministic: dk then dv partials, each [split][lk][heads * HD]
+        const int64_t i = ((int64_t)split * lk + r) * heads * HD + h * HD + 8 * d + 2 * t;
+        *reinterpret_cast<float2*>(part + i) = vk;
+        *reinterpret_cast<float2*>(part + (int64_t)nsplit * lk * heads * HD + i) = vv;
       } else {
         atomicAdd(dstk, vk);
         atomicAdd(dstv, vv);
@@ -736,18 +743,31 @@ __global__ void __launch_bounds__(256, 2) cross_bwd_tc_kernel(const float* __res
                                                               float* __restrict__ dq, float* __restrict__ dk,
                                                               float* __restrict__ dv, int64_t lq, int64_t lk, int heads,
                                                               int64_t keys_per_split, int64_t q_per_split, Strides sd,
-                                                              BwdGrid bg) {
+                                                              BwdGrid bg, float* __restrict__ part_q,
+                                                              float* __restrict__ part_kv) {
   __shared__ __align__(16) BwdSmem sm;
   int b = blockIdx.x;
   const int nq = bg.xq * heads * bg.sq;
   if (b < nq) {
     const int bx = b % bg.xq, h = (b / bg.xq) % heads, split = b / (bg.xq * heads);
-    cross_bwd_dq_tc(sm, bx, h, split, bg.sq, q, k, v, o, d_o, lse, dq, lq, lk, heads, keys_per_split, sd);
+    cross_bwd_dq_tc(sm, bx, h, split, bg.sq, q, k, v, o, d_o, lse, dq, lq, lk, heads, keys_per_split, sd, part_q);
   } else {
     b -= nq;
     const int bx = b % bg.xk, h = (b / bg.xk) % heads, split = b / (bg.xk * heads);
-    cross_bwd_dkv_tc(sm, bx, h, split, bg.sk, q, k, v, o, d_o, lse, dk, dv, lq, lk, heads, q_per_split, sd);
+    cross_bwd_dkv_tc(sm, bx, h, split, bg.sk, q, k, v, o, d_o, lse, dk, dv, lq, lk, heads, q_per_split, sd, part_kv);
   }
+}
+
+// out[r][c] = sum_s part[s][r][c] over the splits in index order (the deterministic backward's combine, one thread per
+// element: no atomics)
+__global__ void __launch_bounds__(256) cross_split_sum_kernel(const float* __restrict__ part, int splits, int64_t rows,
+                                                              int e, float* __restrict__ out, int64_t ld_out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * e) return;
+  const int64_t r = i / e, c = i % e;
+  float acc = 0.f;
+  for (int s = 0; s < splits; ++s) acc += part[(int64_t)s * rows * e + i];
+  out[r * ld_out + c] = acc;
 }
 
 // rows_parallel rows spread over CTAs of `rows_per_cta`, the other side looped in chunks of `chunk`: how many loop splits?
@@ -830,27 +850,51 @@ extern "C" int mt_cross_attn_fwd(const void* q, int64_t ldq, const void* k, cons
   return check_launch("cross_fwd_kernel");
 }
 
-extern "C" int mt_cross_attn_bwd(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* o,
-                                 const void* d_o, int64_t ldo, const float* lse, int dtype, float* dq_f32, int64_t lddq,
-                                 float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads,
-                                 int head_dim, int impl, void* stream) {
+// Plans of the two roles of the backward: tensor-core path: both roles of the one backward kernel run with the same CTA size
+static void bwd_plans(int64_t lq, int64_t lk, int heads, bool tc, int* fw, Plan* pq, Plan* pk) {
+  *fw = tc ? (tc_warps(lq) > tc_warps(lk) ? tc_warps(lq) : tc_warps(lk)) : 0;
+  *pq = make_plan(lq, lk, heads, tc, *fw);
+  *pk = make_plan(lk, lq, heads, tc, *fw);
+}
+
+extern "C" int64_t mt_cross_attn_bwd_workspace_floats(int64_t lq, int64_t lk, int heads, int head_dim, int dtype, int impl) {
+  (void)head_dim;
+  int fw;
+  Plan pq, pk;
+  bwd_plans(lq, lk, heads, use_tc(impl, dtype), &fw, &pq, &pk);
+  const int64_t e = (int64_t)heads * HD;
+  return (pq.splits > 1 ? (int64_t)pq.splits * lq * e : 0) + (pk.splits > 1 ? 2 * (int64_t)pk.splits * lk * e : 0);
+}
+
+static int cross_attn_bwd(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* o,
+                          const void* d_o, int64_t ldo, const float* lse, int dtype, float* dq_f32, int64_t lddq,
+                          float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads, int head_dim,
+                          float* workspace, int64_t workspace_floats, bool deterministic, int impl, cudaStream_t st) {
   MT_REQUIRE(head_dim == HD, "cross_attn: head_dim must be 16 (got %d)", head_dim);
   MT_REQUIRE(lq > 0 && lk > 0 && heads > 0 && heads <= 65535, "cross_attn: bad sizes");
   MT_REQUIRE(impl == 0 || impl == 1, "cross_attn: impl must be 0 (SIMT fp32) or 1 (TF32 tensor cores)");
   const int64_t e = (int64_t)heads * HD;
   MT_REQUIRE(ldq >= e && ldkv >= e && ldo >= e && lddq >= e && lddkv >= e && ((ldq | ldkv | ldo | lddq | lddkv) & 7) == 0,
              "cross_attn_bwd: bad row strides");
-  cudaStream_t st = (cudaStream_t)stream;
   const bool tc = use_tc(impl, dtype);
-  // tensor-core path: both roles of the one backward kernel run with the same CTA size
-  const int fw = tc ? (tc_warps(lq) > tc_warps(lk) ? tc_warps(lq) : tc_warps(lk)) : 0;
-  const Plan pq = make_plan(lq, lk, heads, tc, fw), pk = make_plan(lk, lq, heads, tc, fw);
+  int fw;
+  Plan pq, pk;
+  bwd_plans(lq, lk, heads, tc, &fw, &pq, &pk);
   MT_REQUIRE(((reinterpret_cast<uintptr_t>(dq_f32) | reinterpret_cast<uintptr_t>(dk_f32) |
                reinterpret_cast<uintptr_t>(dv_f32)) & 15) == 0, "cross_attn_bwd: gradients must be 16-byte aligned");
-  // split loops accumulate with vector reduce-adds into zero-filled gradients; an unsplit loop owns its rows and stores
+  if (deterministic) {
+    MT_REQUIRE(tc, "cross_attn_bwd: the deterministic backward is the tensor-core one (impl 1, f32 tensors)");
+    MT_REQUIRE(workspace_floats >= mt_cross_attn_bwd_workspace_floats(lq, lk, heads, head_dim, dtype, impl) &&
+               (workspace != nullptr || workspace_floats == 0) && ((uintptr_t)workspace & 15) == 0,
+               "cross_attn_bwd: workspace too small or not 16-byte aligned");
+  }
+  // split loops accumulate with vector reduce-adds into zero-filled gradients (deterministic: store partials that a
+  // second pass sums in split order); an unsplit loop owns its rows and stores
+  float* part_q = deterministic && pq.splits > 1 ? workspace : nullptr;
+  float* part_kv = deterministic && pk.splits > 1 ? workspace + (pq.splits > 1 ? (int64_t)pq.splits * lq * e : 0) : nullptr;
   const size_t wbytes = sizeof(float) * (size_t)e;
-  if (pq.splits > 1) MT_CUDA(cudaMemset2DAsync(dq_f32, sizeof(float) * lddq, 0, wbytes, (size_t)lq, st));
-  if (pk.splits > 1) {
+  if (pq.splits > 1 && part_q == nullptr) MT_CUDA(cudaMemset2DAsync(dq_f32, sizeof(float) * lddq, 0, wbytes, (size_t)lq, st));
+  if (pk.splits > 1 && part_kv == nullptr) {
     MT_CUDA(cudaMemset2DAsync(dk_f32, sizeof(float) * lddkv, 0, wbytes, (size_t)lk, st));
     MT_CUDA(cudaMemset2DAsync(dv_f32, sizeof(float) * lddkv, 0, wbytes, (size_t)lk, st));
   }
@@ -862,7 +906,20 @@ extern "C" int mt_cross_attn_bwd(const void* q, int64_t ldq, const void* k, cons
     const BwdGrid bg{(int)pq.grid_x, pq.splits, (int)pk.grid_x, pk.splits};
     const unsigned total = (unsigned)((int64_t)bg.xq * heads * bg.sq + (int64_t)bg.xk * heads * bg.sk);
     cross_bwd_tc_kernel<<<total, 32 * fw, 0, st>>>((const f*)q, (const f*)k, (const f*)v, (const f*)o, (const f*)d_o, lse,
-                                                  dq_f32, dk_f32, dv_f32, lq, lk, heads, pq.per_split, pk.per_split, sd, bg);
+                                                  dq_f32, dk_f32, dv_f32, lq, lk, heads, pq.per_split, pk.per_split, sd, bg,
+                                                  part_q, part_kv);
+    if (part_q != nullptr || part_kv != nullptr) {
+      if (int rc = check_launch("cross_bwd_tc_kernel")) return rc;
+      if (part_q != nullptr)
+        cross_split_sum_kernel<<<(unsigned)((lq * e + 255) / 256), 256, 0, st>>>(part_q, pq.splits, lq, (int)e, dq_f32, lddq);
+      if (part_kv != nullptr) {
+        const int64_t n = lk * e;
+        cross_split_sum_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part_kv, pk.splits, lk, (int)e, dk_f32, lddkv);
+        cross_split_sum_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(part_kv + (int64_t)pk.splits * n, pk.splits, lk,
+                                                                            (int)e, dv_f32, lddkv);
+      }
+      return check_launch("cross_split_sum_kernel");
+    }
   } else if (dtype == MT_F32) {
     using f = float;
     cross_bwd_dq_kernel<f><<<gq, XT, 0, st>>>((const f*)q, (const f*)k, (const f*)v, (const f*)o, (const f*)d_o, lse,
@@ -880,4 +937,20 @@ extern "C" int mt_cross_attn_bwd(const void* q, int64_t ldq, const void* k, cons
     return MT_E_BADARG;
   }
   return check_launch("cross_bwd kernels");
+}
+
+extern "C" int mt_cross_attn_bwd(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* o,
+                                 const void* d_o, int64_t ldo, const float* lse, int dtype, float* dq_f32, int64_t lddq,
+                                 float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads,
+                                 int head_dim, int impl, void* stream) {
+  return cross_attn_bwd(q, ldq, k, v, ldkv, o, d_o, ldo, lse, dtype, dq_f32, lddq, dk_f32, dv_f32, lddkv, lq, lk, heads,
+                        head_dim, nullptr, 0, false, impl, (cudaStream_t)stream);
+}
+
+extern "C" int mt_cross_attn_bwd_ws(const void* q, int64_t ldq, const void* k, const void* v, int64_t ldkv, const void* o,
+                                    const void* d_o, int64_t ldo, const float* lse, int dtype, float* dq_f32, int64_t lddq,
+                                    float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads,
+                                    int head_dim, float* workspace, int64_t workspace_floats, int impl, void* stream) {
+  return cross_attn_bwd(q, ldq, k, v, ldkv, o, d_o, ldo, lse, dtype, dq_f32, lddq, dk_f32, dv_f32, lddkv, lq, lk, heads,
+                        head_dim, workspace, workspace_floats, true, impl, (cudaStream_t)stream);
 }

@@ -953,6 +953,10 @@ __device__ __forceinline__ void stage_chunk(uint8_t* stg, int row, int c, float4
   *reinterpret_cast<float4*>(dst) = v;
 }
 
+// WITH_DQ = false (impl 4, the deterministic backward): dK / dV only -- no dQ MMA, no dS^T shared-memory tile (it only
+// feeds that MMA) and idle drain warps; dQ comes from dilated_bwd_dq_sm100_kernel.  Every key slot of a branch belongs to
+// exactly one key tile, so its dK / dV rows receive one non-zero reduce-add per launch.
+template <bool WITH_DQ>
 __global__ void __launch_bounds__(BWD3_THREADS, 1)
 dilated_bwd_sm100_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ TensorMaps do_maps,
                           const __grid_constant__ TensorMaps dq32_maps, const __grid_constant__ TensorMaps dq16_maps,
@@ -1167,7 +1171,7 @@ dilated_bwd_sm100_kernel(const __grid_constant__ TensorMaps maps, const __grid_c
         MT_TRACE(200 + g);
         issue_st(std::integral_constant<int, 2 * st2 + hh>{});
       }
-      if (hh == 1) {                 // both halves of query tile i are done: dQ_i = dS_i K
+      if (WITH_DQ && hh == 1) {      // both halves of query tile i are done: dQ_i = dS_i K
         if (i > 0) mbar_wait(bar_dq_free, (i - 1) & 1);
         tc_fence_after();
         MT_TRACE(300 + g);
@@ -1256,8 +1260,10 @@ dilated_bwd_sm100_kernel(const __grid_constant__ TensorMaps maps, const __grid_c
       tmem_st8(ts, pk);
       tmem_st8(td, dk);
       // dS^T half tile for dQ = dS K: [key row][64 queries] block hh, 16 queries = 2 swizzled 16-byte chunks
-      *reinterpret_cast<uint4*>(drow + (((2 * qq) ^ sw) << 4)) = make_uint4(dk[0], dk[1], dk[2], dk[3]);
-      *reinterpret_cast<uint4*>(drow + (((2 * qq + 1) ^ sw) << 4)) = make_uint4(dk[4], dk[5], dk[6], dk[7]);
+      if constexpr (WITH_DQ) {
+        *reinterpret_cast<uint4*>(drow + (((2 * qq) ^ sw) << 4)) = make_uint4(dk[0], dk[1], dk[2], dk[3]);
+        *reinterpret_cast<uint4*>(drow + (((2 * qq + 1) ^ sw) << 4)) = make_uint4(dk[4], dk[5], dk[6], dk[7]);
+      }
       tmem_st_wait();
       fence_proxy_async_smem();
       tc_fence_before();
@@ -1298,7 +1304,7 @@ dilated_bwd_sm100_kernel(const __grid_constant__ TensorMaps maps, const __grid_c
     }
     MT_TRACE(6);
     if (warp == 0 && lane == 0) { MT_TRACE_DUMP("cmp3"); }
-  } else {
+  } else if constexpr (WITH_DQ) {
     // ===== dQ drain (4 warps, one query row per thread) ================================================================
     const int lane_grp = warp & 3;
     const int row = lane_grp * 32 + lane;
@@ -1994,6 +2000,299 @@ dilated_bwd_sm100_persistent_kernel(const __grid_constant__ TensorMaps maps, con
 #endif
 }
 
+// =====================================================================================================================
+// backward, deterministic (impl 4): dQ query tile by query tile
+// =====================================================================================================================
+// One CTA = one (branch, segment, head, 128-slot query tile) -- the pipeline of dilated_fwd_sm100_k48_kernel with the dO
+// tile and a second score MMA.  Per 48-key tile of the segment:
+//   S = Q K^T and dP = dO V^T into TMEM (SS MMAs, N = 48);
+//   P = exp2(S scale log2e - lse log2e) with the FINAL merged lse: no running maximum and no rescale;
+//   dS = P (dP - delta_b), packed to bf16 pairs in TMEM;
+//   dQ += dS K: a TS MMA with K as the MN-major B operand, the way the forward uses P and V.
+// A query row is a TMEM lane, so lse and delta are one scalar per thread.  dQ * scale leaves once per tile: the thread of
+// a row adds it to that row of dqkv, a plain load-add-store, because no other CTA of the launch touches the element.
+// Rows of the tile that are not its queries (slots >= m belong to the next segment, positions >= N are padding) are
+// not written at all: their S against this segment's keys is not zero, so they are given P = 0 and skipped.
+// TMEM: S [0,48) | dP [48,96) | dS (bf16 pairs) [96,120) | dQ [128,176) -> a 256-column allocation (two CTAs per SM).
+// Shared memory: Q + dO tiles (32 KB) and a four-stage ring of 48-key K / V tiles (48 KB): 80 KB, so at most two CTAs
+// share an SM, the number the TMEM allocation allows.
+static constexpr int DQ_KS = 4;                   // K / V ring stages
+static constexpr uint32_t TMEM_DQ_COLS = 256;
+struct BwdDqSmem {
+  static constexpr int Q = 0;
+  static constexpr int DO = Q + TILE_BYTES;
+  static constexpr int K = DO + TILE_BYTES;
+  static constexpr int V = K + DQ_KS * KT_BYTES;
+  static constexpr int BAR = V + DQ_KS * KT_BYTES;
+  // barriers (8 B each): qdo_full, s_full, s_free, p_full, dq_full, kv_full[DQ_KS], kv_empty[DQ_KS]; the TMEM pointer
+  static constexpr int NBAR = 5 + 2 * DQ_KS;
+  static constexpr int TMEM_PTR = BAR + NBAR * 8;
+  static constexpr int TOTAL = TMEM_PTR + 16;
+};
+static_assert(KT == 48, "the dQ kernel's TMEM layout is laid out for 48-key tiles");
+
+__global__ void __launch_bounds__(FWD_THREADS, 2)
+dilated_bwd_dq_sm100_kernel(const __grid_constant__ TensorMaps maps, const __grid_constant__ TensorMaps kv_maps,
+                            const __grid_constant__ TensorMaps do_maps, const Sm100Params P,
+                            const float* __restrict__ lse, const float* __restrict__ delta_br, float* __restrict__ dqkv) {
+  extern __shared__ __align__(1024) uint8_t smem[];
+  const uint32_t sbase = smem_u32(smem);
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  constexpr int W_TMA = 4, W_MMA = 5;
+  if ((sbase & 1023u) != 0) {
+    __trap();
+  }
+  int oi = 0;
+  while (oi + 1 < P.geo.nb && (int)blockIdx.x >= P.item_prefix[oi + 1]) ++oi;
+  const int b = P.order[oi];
+  const BranchGeom bg = P.geo.b[b];
+  int local = blockIdx.x - P.item_prefix[oi];
+  const int qt = local % P.tiles[b];
+  local /= P.tiles[b];
+  const int h = local % P.geo.H;
+  const int s = local / P.geo.H;
+  const int H = P.geo.H, N = P.geo.N, E = H * DH;
+  const int off = (h * bg.r) / H;
+  const int jseg = (s * bg.g) / bg.r;
+  const int q0 = qt * BT;
+  const int seg_lo = s * bg.g + off;
+  const int seg_end = min(N, (s + 1) * bg.g);
+  const int c_real = seg_end > seg_lo ? (seg_end - seg_lo + bg.r - 1) / bg.r : 0;
+  if (q0 >= c_real) return;                                   // a tile of padding queries only
+  const int n_kv = min((bg.m + KT - 1) / KT, (c_real + KT - 1) / KT);   // key tiles of padding only have K = 0
+
+  const uint32_t bar_qdo_full = sbase + BwdDqSmem::BAR + 0;
+  const uint32_t bar_s_full = sbase + BwdDqSmem::BAR + 8;
+  const uint32_t bar_s_free = sbase + BwdDqSmem::BAR + 16;
+  const uint32_t bar_p_full = sbase + BwdDqSmem::BAR + 24;
+  const uint32_t bar_dq_full = sbase + BwdDqSmem::BAR + 32;
+  const uint32_t bar_kv_full = sbase + BwdDqSmem::BAR + 40;   // [DQ_KS]
+  const uint32_t bar_kv_empty = bar_kv_full + 8 * DQ_KS;      // [DQ_KS]
+  volatile uint32_t* tmem_slot = reinterpret_cast<volatile uint32_t*>(smem + BwdDqSmem::TMEM_PTR);
+
+  if (threadIdx.x == 0) {
+    mbar_init(bar_qdo_full, 1);
+    for (int i = 0; i < DQ_KS; ++i) {
+      mbar_init(bar_kv_full + 8 * i, 1);
+      mbar_init(bar_kv_empty + 8 * i, 1);
+    }
+    mbar_init(bar_s_full, 1);
+    mbar_init(bar_s_free, 128);
+    mbar_init(bar_p_full, 128);
+    mbar_init(bar_dq_full, 1);
+    fence_barrier_init();
+    tma_prefetch_desc(&maps.m[b]);
+    tma_prefetch_desc(&kv_maps.m[b]);
+    tma_prefetch_desc(&do_maps.m[b]);
+  }
+  if (warp == W_MMA) {
+    tmem_alloc(smem_u32((const void*)tmem_slot), TMEM_DQ_COLS);
+    tmem_relinquish();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  const uint32_t tmem = *tmem_slot;
+  const uint32_t tmem_s = tmem, tmem_dp = tmem + KT, tmem_ds = tmem + 2 * KT, tmem_dq = tmem + 128;
+
+  if (warp == W_TMA) {
+    // ===== TMA producer ===============================================================================================
+    if (lane == 0) {
+      const void* kmap = &kv_maps.m[b];    // the qkv view with a 48-slot box
+      mbar_expect_tx(bar_qdo_full, 2 * TILE_BYTES);
+      tma_load_3d(sbase + BwdDqSmem::Q, &maps.m[b], bar_qdo_full, h * DH, off, jseg + q0);
+      tma_load_3d(sbase + BwdDqSmem::DO, &do_maps.m[b], bar_qdo_full, h * DH, off, jseg + q0);
+      for (int j = 0; j < n_kv; ++j) {
+        const int st = j % DQ_KS, use = j / DQ_KS;
+        mbar_wait(bar_kv_empty + 8 * st, (use & 1) ^ 1);
+        mbar_expect_tx(bar_kv_full + 8 * st, 2 * KT_BYTES);
+        tma_load_3d(sbase + BwdDqSmem::K + st * KT_BYTES, kmap, bar_kv_full + 8 * st, E + h * DH, off, jseg + j * KT);
+        tma_load_3d(sbase + BwdDqSmem::V + st * KT_BYTES, kmap, bar_kv_full + 8 * st, 2 * E + h * DH, off, jseg + j * KT);
+      }
+    }
+  } else if (warp == W_MMA) {
+    // ===== MMA issuer =================================================================================================
+    constexpr uint32_t IDESC_S = umma_idesc_bf16(BT, KT, 0, 0);    // S, dP: A = Q / dO, B = K / V (both K-major)
+    constexpr uint32_t IDESC_DQ = umma_idesc_bf16(BT, DH, 0, 1);   // dQ: A = dS (TMEM), B = K (MN-major)
+    const uint64_t q_desc = umma_smem_desc(sbase + BwdDqSmem::Q, 16, 1024);
+    const uint64_t do_desc = umma_smem_desc(sbase + BwdDqSmem::DO, 16, 1024);
+    const uint64_t k_desc0 = umma_smem_desc(sbase + BwdDqSmem::K, 16, 1024);
+    const uint64_t v_desc0 = umma_smem_desc(sbase + BwdDqSmem::V, 16, 1024);
+    const uint64_t kmn_desc0 = umma_smem_desc(sbase + BwdDqSmem::K, KT_BYTES, 1024);
+    auto issue_s = [&](int j) {   // S_j = Q K_j^T and dP_j = dO V_j^T: three k-steps of 16 each
+      if (elect_one()) {
+        const uint32_t so = (uint32_t)(j % DQ_KS) * KT_BYTES;
+        const uint64_t kd = umma_desc_adv(k_desc0, so), vd = umma_desc_adv(v_desc0, so);
+#pragma unroll
+        for (int k = 0; k < DH / 16; ++k)
+          umma_ss(tmem_s, umma_desc_adv(q_desc, k * 32), umma_desc_adv(kd, k * 32), IDESC_S, k > 0);
+#pragma unroll
+        for (int k = 0; k < DH / 16; ++k)
+          umma_ss(tmem_dp, umma_desc_adv(do_desc, k * 32), umma_desc_adv(vd, k * 32), IDESC_S, k > 0);
+        umma_commit(bar_s_full);
+      }
+      __syncwarp();
+    };
+    mbar_wait(bar_qdo_full, 0);
+    mbar_wait(bar_kv_full, 0);
+    tc_fence_after();
+    issue_s(0);
+    for (int j = 0; j < n_kv; ++j) {
+      if (j + 1 < n_kv) {
+        mbar_wait(bar_kv_full + 8 * ((j + 1) % DQ_KS), ((j + 1) / DQ_KS) & 1);
+        mbar_wait(bar_s_free, j & 1);   // S_j and dP_j are in registers
+        tc_fence_after();
+        issue_s(j + 1);
+      }
+      mbar_wait(bar_p_full, j & 1);     // dS_j is in TMEM
+      tc_fence_after();
+      if (elect_one()) {
+        const uint64_t kd = umma_desc_adv(kmn_desc0, (uint32_t)(j % DQ_KS) * KT_BYTES);
+#pragma unroll
+        for (int k = 0; k < KT / 16; ++k)   // 16 keys = 8 packed dS columns = 16 rows of the K tile (2048 B)
+          umma_ts(tmem_dq, tmem_ds + k * 8, umma_desc_adv(kd, k * 2048), IDESC_DQ, (j > 0) || (k > 0));
+        umma_commit(bar_kv_empty + 8 * (j % DQ_KS));
+        umma_commit(bar_dq_full);
+      }
+      __syncwarp();
+    }
+  } else {
+    // ===== dS: one query row per thread =================================================================================
+    const int lane_grp = warp & 3;
+    const int row = lane_grp * 32 + lane;
+    const uint32_t t_lane = (uint32_t)(lane_grp * 32) << 16;
+    const int slot = q0 + row;
+    const int pos = seg_lo + slot * bg.r;
+    const bool qok = slot < bg.m && pos < seg_end;     // this tile's own query
+    const int slot_h = h - off * bg.hpb;
+    const float lb = qok ? lse[(int64_t)pos * H + h] * 1.4426950408889634f : INFINITY;   // +inf: P = 0
+    const float dl = qok ? delta_br[bg.lse_off + (int64_t)pos * bg.hpb + slot_h] : 0.f;
+    const float scale_log2 = P.scale_log2;
+    auto tile = [&](int j, auto mask_tag) {
+      constexpr bool MASK = decltype(mask_tag)::value;
+      const int kvalid = bg.m - j * KT;  // key slots of this tile that belong to the segment
+      mbar_wait(bar_s_full, j & 1);
+      tc_fence_after();
+      float sv[KT], dp[KT];
+      {
+        float lo[32], hi[16], dlo[32], dhi[16];
+        tmem_ld32(tmem_s + t_lane, lo);
+        tmem_ld16(tmem_s + t_lane + 32, hi);
+        tmem_ld32(tmem_dp + t_lane, dlo);
+        tmem_ld16(tmem_dp + t_lane + 32, dhi);
+        tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 32; ++i) { sv[i] = lo[i]; dp[i] = dlo[i]; }
+#pragma unroll
+        for (int i = 0; i < 16; ++i) { sv[32 + i] = hi[i]; dp[32 + i] = dhi[i]; }
+      }
+      tc_fence_before();
+      mbar_arrive(bar_s_free);           // the MMA warp may overwrite S / dP with tile j + 1
+      if (j > 0) {                       // dS_j overwrites dS_{j-1}: its dQ MMA must have read it
+        mbar_wait(bar_dq_full, (j - 1) & 1);
+        tc_fence_after();
+      }
+#pragma unroll
+      for (int c = 0; c < KT / 16; ++c) {
+        uint32_t pk[8];
+#pragma unroll
+        for (int i = 0; i < 16; i += 2) {
+          const int k = c * 16 + i;
+          float p0 = ex2(fmaf(sv[k], scale_log2, -lb));
+          float p1 = ex2(fmaf(sv[k + 1], scale_log2, -lb));
+          if (MASK) {
+            p0 = k < kvalid ? p0 : 0.f;
+            p1 = k + 1 < kvalid ? p1 : 0.f;
+          }
+          pk[i >> 1] = pack_bf16(p0 * (dp[k] - dl), p1 * (dp[k + 1] - dl));
+        }
+        tmem_st8(tmem_ds + t_lane + c * 8, pk);
+      }
+      tmem_st_wait();
+      tc_fence_before();
+      mbar_arrive(bar_p_full);
+    };
+    for (int j = 0; j < n_kv; ++j) {
+      if (bg.m - j * KT >= KT) tile(j, std::false_type{});
+      else tile(j, std::true_type{});
+    }
+    mbar_wait(bar_dq_full, (n_kv - 1) & 1);
+    tc_fence_after();
+    float lo[32], hi[16];
+    tmem_ld32(tmem_dq + t_lane, lo);
+    tmem_ld16(tmem_dq + t_lane + 32, hi);
+    tmem_ld_wait();
+    if (qok) {
+      const float sc = P.scale;
+      float* dst = dqkv + (int64_t)pos * 3 * E + h * DH;
+#pragma unroll
+      for (int c = 0; c < DH / 4; ++c) {
+        float4 a = *reinterpret_cast<const float4*>(dst + 4 * c);
+        const float* v = c < 8 ? lo + 4 * c : hi + 4 * (c - 8);
+        // product and sum rounded separately (no FMA contraction): the branch's value is v * sc whatever came before
+        a.x = __fadd_rn(a.x, __fmul_rn(v[0], sc));
+        a.y = __fadd_rn(a.y, __fmul_rn(v[1], sc));
+        a.z = __fadd_rn(a.z, __fmul_rn(v[2], sc));
+        a.w = __fadd_rn(a.w, __fmul_rn(v[3], sc));
+        *reinterpret_cast<float4*>(dst + 4 * c) = a;
+      }
+    }
+  }
+  tc_fence_before();
+  __syncthreads();
+  if (warp == W_MMA) tmem_dealloc(tmem, TMEM_DQ_COLS);
+}
+
+// The launch parameters of ONE branch b of P: item i of the launch is item i of branch b.
+static Sm100Params branch_only(const Sm100Params& P, int b) {
+  Sm100Params Q = P;
+  Q.order[0] = b;
+  Q.item_prefix[0] = 0;
+  for (int i = 1; i <= P.geo.nb; ++i) Q.item_prefix[i] = P.geo.b[b].n_seg * P.geo.H * P.tiles[b];
+  return Q;
+}
+
+// impl 4.  Why the result is the same in every run:
+//   * dqkv is zeroed by the caller (mt_dilated_attn_bwd); then the branches run one after another on the stream, branch
+//     b = 0, 1, ..., nb - 1, each as two launches: dQ (dilated_bwd_dq_sm100_kernel) and dK / dV
+//     (dilated_bwd_sm100_kernel<false>).  Stream order fixes the order in which the branches are added.
+//   * Within one launch every element receives at most ONE non-zero addition: a (position, head) of a branch belongs to
+//     exactly one (segment, head, slot), hence to one query tile (dQ: written by the thread of its row) and to one key
+//     tile (dK / dV: one TMA reduce-add by the CTA of that tile).
+//   * The only other additions are the +0.0 rows a key tile carries past its segment's m (the next segment's keys, masked
+//     to P = 0).  Adding +0.0 gives the same bits in either order: x + 0 = x for x != -0, and the sum comes out +0 both
+//     ways when it is zero.
+// No CTA waits for another: the order comes from the stream, never from counters or spinning.
+static int dilated_attn_bwd_deterministic(const Sm100Params& P, const TensorMaps& maps, const TensorMaps& do_maps,
+                                          const TensorMaps& dq32_maps, const TensorMaps& dq16_maps, const void* qkv,
+                                          int64_t qkv_ld, int64_t n_alloc, const float* lse, const float* delta_br,
+                                          float* dqkv, cudaStream_t st) {
+  TensorMaps kv_maps;
+  memset(&kv_maps, 0, sizeof(kv_maps));
+  for (int b = 0; b < P.geo.nb; ++b) {
+    const int rc = encode_branch_map(&kv_maps.m[b], qkv, qkv_ld, n_alloc, P.geo.b[b].r, KT);
+    if (rc) return rc;
+  }
+  static bool attr_set = false;   // once per process: the call is not free and never changes
+  if (!attr_set) {
+    MT_CUDA(cudaFuncSetAttribute(dilated_bwd_dq_sm100_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, BwdDqSmem::TOTAL));
+    MT_CUDA(cudaFuncSetAttribute(dilated_bwd_sm100_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, Bwd3Smem::TOTAL));
+    attr_set = true;
+  }
+  for (int b = 0; b < P.geo.nb; ++b) {
+    const Sm100Params Pb = branch_only(P, b);
+    const int items = Pb.item_prefix[1];
+    if (items == 0) continue;
+    dilated_bwd_dq_sm100_kernel<<<items, FWD_THREADS, BwdDqSmem::TOTAL, st>>>(maps, kv_maps, do_maps, Pb, lse, delta_br,
+                                                                              dqkv);
+    if (int rc = check_launch("dilated_bwd_dq_sm100_kernel")) return rc;
+    dilated_bwd_sm100_kernel<false><<<items, BWD3_THREADS, Bwd3Smem::TOTAL, st>>>(maps, do_maps, dq32_maps, dq16_maps, Pb,
+                                                                                  lse, delta_br);
+    if (int rc = check_launch("dilated_bwd_sm100_kernel<false>")) return rc;
+  }
+  return 0;
+}
+
 int dilated_attn_bwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
                            const void* dattn, const float* lse, const float* delta_br, float* dqkv, int impl,
                            cudaStream_t st) {
@@ -2035,14 +2334,16 @@ int dilated_attn_bwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int
                                                                                     lse, delta_br, counter);
     return check_launch("dilated_bwd_sm100_persistent_kernel");
   }
+  if (impl == 4) return dilated_attn_bwd_deterministic(P, maps, do_maps, dq32_maps, dq16_maps, qkv, qkv_ld, n_alloc, lse,
+                                                      delta_br, dqkv, st);
   {
     static bool attr_set = false;   // once per process: the call is not free and never changes
     if (!attr_set) {
-      MT_CUDA(cudaFuncSetAttribute(dilated_bwd_sm100_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Bwd3Smem::TOTAL));
+      MT_CUDA(cudaFuncSetAttribute(dilated_bwd_sm100_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, Bwd3Smem::TOTAL));
       attr_set = true;
     }
   }
-  dilated_bwd_sm100_kernel<<<P.item_prefix[P.geo.nb], BWD3_THREADS, Bwd3Smem::TOTAL, st>>>(
+  dilated_bwd_sm100_kernel<true><<<P.item_prefix[P.geo.nb], BWD3_THREADS, Bwd3Smem::TOTAL, st>>>(
       maps, do_maps, dq32_maps, dq16_maps, P, lse, delta_br);
   return check_launch("dilated_bwd_sm100_kernel");
 }

@@ -201,7 +201,8 @@ __global__ void __launch_bounds__(RowCfg<COLS>::THREADS, RowCfg<COLS>::MINB) ln_
                                                      const float* __restrict__ gamma, const float* __restrict__ mean,
                                                      const float* __restrict__ rstd, const TR* __restrict__ residual,
                                                      TDX* __restrict__ dx, __nv_bfloat16* __restrict__ dx_lp,
-                                                     float* __restrict__ dgamma, float* __restrict__ dbeta, int64_t rows) {
+                                                     float* __restrict__ dgamma, float* __restrict__ dbeta, int64_t rows,
+                                                     float* __restrict__ part) {
   using C = RowCfg<COLS>;
   __shared__ float red[C::RPB * (C::TPR / 32) + 1];
   const int t = threadIdx.x % C::TPR, rib = threadIdx.x / C::TPR;
@@ -284,6 +285,28 @@ __global__ void __launch_bounds__(RowCfg<COLS>::THREADS, RowCfg<COLS>::MINB) ln_
     // the RPB row-lanes of the block hold partials for the same columns: combine them in shared memory first, so that
     // every column receives ONE global atomic per block (same-address atomics serialise in L2)
     __shared__ float wsum[2 * COLS];
+    if (part != nullptr) {
+      // deterministic: the row-lanes add their partials in index order, the block's sums go to part[0 / 1][block][COLS]
+      // and colsum_partials_kernel adds the blocks in index order
+      for (int r = 0; r < C::RPB; ++r) {
+        if (rib == r) {
+#pragma unroll
+          for (int i = 0; i < C::NCH; ++i)
+#pragma unroll
+            for (int j = 0; j < 8; ++j) {
+              const int c = (i * C::TPR + t) * 8 + j;
+              wsum[c] = r == 0 ? dg_acc[i][j] : wsum[c] + dg_acc[i][j];
+              wsum[COLS + c] = r == 0 ? db_acc[i][j] : wsum[COLS + c] + db_acc[i][j];
+            }
+        }
+        __syncthreads();
+      }
+      for (int c = threadIdx.x; c < COLS; c += blockDim.x) {
+        part[(int64_t)blockIdx.x * COLS + c] = wsum[c];
+        part[(int64_t)(gridDim.x + blockIdx.x) * COLS + c] = wsum[COLS + c];
+      }
+      return;
+    }
     for (int c = threadIdx.x; c < 2 * COLS; c += blockDim.x) wsum[c] = 0.f;
     __syncthreads();
 #pragma unroll
@@ -449,7 +472,8 @@ __global__ void __launch_bounds__(768) gated_residual_bwd_kernel(const float* __
                                                                  const TB* __restrict__ b,
                                                                  const float* __restrict__ gate, float* __restrict__ da,
                                                                  TB* __restrict__ db, float* __restrict__ dgate,
-                                                                 float* __restrict__ dysum, int64_t rows, int cols) {
+                                                                 float* __restrict__ dysum, int64_t rows, int cols,
+                                                                 float* __restrict__ part) {
   // thread t owns column chunk (t % chunks) for rows (blockIdx.x * rpb + t / chunks) + k * gridDim.x * rpb;
   // blockDim.x == chunks * rpb
   extern __shared__ float gr_red[];
@@ -493,6 +517,12 @@ __global__ void __launch_bounds__(768) gated_residual_bwd_kernel(const float* __
       for (int r = 0; r + 1 < rpb; ++r) {
 #pragma unroll
         for (int j = 0; j < 8; ++j) acc[j] += gr_red[(r * chunks + ch) * 8 + j];
+      }
+      if (part != nullptr) {   // deterministic: part[pass][block][cols], summed in block order by colsum_partials_kernel
+        float4* dst = reinterpret_cast<float4*>(part + ((int64_t)pass * gridDim.x + blockIdx.x) * cols + ch * 8);
+        dst[0] = make_float4(acc[0], acc[1], acc[2], acc[3]);
+        dst[1] = make_float4(acc[4], acc[5], acc[6], acc[7]);
+        continue;
       }
       float4* dst = reinterpret_cast<float4*>((pass == 0 ? dgate : dysum) + ch * 8);
       atomicAdd(dst, make_float4(acc[0], acc[1], acc[2], acc[3]));
@@ -594,7 +624,7 @@ ffn_bwd_prep_kernel(const float* __restrict__ dy, const float* __restrict__ y, c
 // out[c] = sum_r x[r, c] (bias gradients of the adapter's projections): float4 column quads, RL row lanes per block,
 // shared-memory combine, ONE 16-byte reduce-add per column quad and block into the zeroed output
 __global__ void __launch_bounds__(1024) colsum_kernel(const float* __restrict__ x, int64_t ld, float* __restrict__ out,
-                                                      int64_t rows, int quads, int row_lanes) {
+                                                      int64_t rows, int quads, int row_lanes, float4* __restrict__ part) {
   extern __shared__ float4 cs_red[];
   const int qd = threadIdx.x % quads, rl = threadIdx.x / quads;
   float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
@@ -612,8 +642,22 @@ __global__ void __launch_bounds__(1024) colsum_kernel(const float* __restrict__ 
       const float4 v = cs_red[i * quads + qd];
       acc.x += v.x; acc.y += v.y; acc.z += v.z; acc.w += v.w;
     }
-    atomicAdd(reinterpret_cast<float4*>(out) + qd, acc);
+    if (part != nullptr) part[(int64_t)blockIdx.x * quads + qd] = acc;   // deterministic: summed by colsum_partials_kernel
+    else atomicAdd(reinterpret_cast<float4*>(out) + qd, acc);
   }
+}
+
+// Second pass of the deterministic column reductions: out0[c] = sum_b part[b][c] over the nblk block partials in index
+// order (and out1 from the next nblk rows when it is not NULL).  One thread per column: a fixed order, no atomics.
+__global__ void __launch_bounds__(256) colsum_partials_kernel(const float* __restrict__ part, int nblk, int cols,
+                                                              float* __restrict__ out0, float* __restrict__ out1) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  const int which = blockIdx.y;
+  if (c >= cols) return;
+  const float* p = part + (int64_t)which * nblk * cols + c;
+  float acc = 0.f;
+  for (int b = 0; b < nblk; ++b) acc += p[(int64_t)b * cols];
+  (which == 0 ? out0 : out1)[c] = acc;
 }
 
 // LayerNorm(768) backward of the pre-attention LN (+ residual gradient, + bf16 twin) that ALSO prepares the FFN backward of
@@ -718,13 +762,24 @@ static int dispatch_ln_fwd(const void* x, int xd, const float* xbias, const floa
   return MT_E_UNSUPPORTED;
 }
 
+// The column-reducing kernels (LayerNorm dgamma / dbeta, gated-residual dgate / dysum, colsum) run at most this many
+// blocks; their deterministic variants write one partial row per block and output (mt_colreduce_workspace_floats).
+static constexpr int kColReduceBlocks = 2 * kNumSMs;
+
+// out0 (and out1) = the block partials of `part` summed in block order
+static int sum_partials(const float* part, int nblk, int cols, float* out0, float* out1, cudaStream_t st) {
+  const dim3 grid((unsigned)((cols + 255) / 256), out1 != nullptr ? 2u : 1u);
+  colsum_partials_kernel<<<grid, 256, 0, st>>>(part, nblk, cols, out0, out1);
+  return check_launch("colsum_partials_kernel");
+}
+
 template <int COLS, bool GELU, typename TDY, typename TX, typename TDX>
 static int launch_ln_bwd(const void* dy, const void* x, const float* xbias, const float* gamma, const float* mean, const float* rstd,
                          const void* residual, int rd, void* dx, void* dx_lp, float* dgamma, float* dbeta, int64_t rows,
-                         cudaStream_t st) {
+                         float* part, cudaStream_t st) {
   using C = RowCfg<COLS>;
   int grid = grid_for(rows, C::RPB);
-  if (dgamma != nullptr && grid > kNumSMs * 2) grid = kNumSMs * 2;  // bound the number of atomic flushes
+  if (dgamma != nullptr && grid > kColReduceBlocks) grid = kColReduceBlocks;  // bound the number of atomic flushes
   if (dgamma != nullptr) {
     if constexpr (!GELU) {
       if (residual != nullptr && rd != MT_F32) {
@@ -732,23 +787,27 @@ static int launch_ln_bwd(const void* dy, const void* x, const float* xbias, cons
         return MT_E_UNSUPPORTED;
       }
       ln_bwd_kernel<COLS, TDY, TX, float, TDX, GELU, true><<<grid, C::THREADS, 0, st>>>(
-          (const TDY*)dy, (const TX*)x, xbias, gamma, mean, rstd, (const float*)residual, (TDX*)dx, (__nv_bfloat16*)dx_lp, dgamma, dbeta, rows);
+          (const TDY*)dy, (const TX*)x, xbias, gamma, mean, rstd, (const float*)residual, (TDX*)dx, (__nv_bfloat16*)dx_lp, dgamma, dbeta, rows, part);
+      if (part != nullptr) {
+        if (int rc = check_launch("ln_bwd_kernel")) return rc;
+        return sum_partials(part, grid, COLS, dgamma, dbeta, st);
+      }
     }
   } else if (residual == nullptr || rd == MT_F32)
     ln_bwd_kernel<COLS, TDY, TX, float, TDX, GELU, false><<<grid, C::THREADS, 0, st>>>(
-        (const TDY*)dy, (const TX*)x, xbias, gamma, mean, rstd, (const float*)residual, (TDX*)dx, (__nv_bfloat16*)dx_lp, dgamma, dbeta, rows);
+        (const TDY*)dy, (const TX*)x, xbias, gamma, mean, rstd, (const float*)residual, (TDX*)dx, (__nv_bfloat16*)dx_lp, dgamma, dbeta, rows, nullptr);
   else
     ln_bwd_kernel<COLS, TDY, TX, __nv_bfloat16, TDX, GELU, false><<<grid, C::THREADS, 0, st>>>(
-        (const TDY*)dy, (const TX*)x, xbias, gamma, mean, rstd, (const __nv_bfloat16*)residual, (TDX*)dx, (__nv_bfloat16*)dx_lp, dgamma, dbeta, rows);
+        (const TDY*)dy, (const TX*)x, xbias, gamma, mean, rstd, (const __nv_bfloat16*)residual, (TDX*)dx, (__nv_bfloat16*)dx_lp, dgamma, dbeta, rows, nullptr);
   return check_launch("ln_bwd_kernel");
 }
 
 template <int COLS, bool GELU>
 static int dispatch_ln_bwd(const void* dy, int dyd, const void* x, int xd, const float* xbias, const float* gamma, const float* mean,
                            const float* rstd, const void* residual, int rd, void* dx, int dxd, void* dx_lp, float* dgamma,
-                           float* dbeta, int64_t rows, cudaStream_t st) {
+                           float* dbeta, int64_t rows, cudaStream_t st, float* part = nullptr) {
 #define MT_LNB(TDY, TX, TDX) \
-  return launch_ln_bwd<COLS, GELU, TDY, TX, TDX>(dy, x, xbias, gamma, mean, rstd, residual, rd, dx, dx_lp, dgamma, dbeta, rows, st)
+  return launch_ln_bwd<COLS, GELU, TDY, TX, TDX>(dy, x, xbias, gamma, mean, rstd, residual, rd, dx, dx_lp, dgamma, dbeta, rows, part, st)
   using bf = __nv_bfloat16;
   if (dyd == MT_F32 && xd == MT_F32 && dxd == MT_F32) MT_LNB(float, float, float);
   if (dyd == MT_BF16 && xd == MT_F32 && dxd == MT_F32) MT_LNB(bf, float, float);
@@ -795,19 +854,37 @@ extern "C" int mt_layernorm_fwd(const void* x, int x_dtype, const float* gamma, 
   return MT_E_UNSUPPORTED;
 }
 
+extern "C" int64_t mt_colreduce_workspace_floats(int64_t cols) { return 2 * (int64_t)kColReduceBlocks * cols; }
+
+static int layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma, const float* mean,
+                         const float* rstd, const void* residual, int res_dtype, void* dx, int dx_dtype, void* dx_bf16,
+                         float* dgamma, float* dbeta, int64_t rows, int64_t cols, float* part, cudaStream_t st) {
+  if (rows == 0) return 0;
+  MT_REQUIRE((dgamma == nullptr) == (dbeta == nullptr), "layernorm bwd: dgamma and dbeta go together");
+  if (cols == 768)
+    return dispatch_ln_bwd<768, false>(dy, dy_dtype, x, x_dtype, nullptr, gamma, mean, rstd, residual, res_dtype, dx, dx_dtype, dx_bf16, dgamma, dbeta, rows, st, part);
+  if (cols == 3072)
+    return dispatch_ln_bwd<3072, false>(dy, dy_dtype, x, x_dtype, nullptr, gamma, mean, rstd, residual, res_dtype, dx, dx_dtype, dx_bf16, dgamma, dbeta, rows, st, part);
+  set_error("layernorm bwd: width %lld not supported (768, 3072)", (long long)cols);
+  return MT_E_UNSUPPORTED;
+}
+
 extern "C" int mt_layernorm_bwd(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma,
                                 const float* mean, const float* rstd, const void* residual, int res_dtype, void* dx,
                                 int dx_dtype, void* dx_bf16, float* dgamma, float* dbeta, int64_t rows, int64_t cols,
                                 void* stream) {
-  cudaStream_t st = (cudaStream_t)stream;
-  if (rows == 0) return 0;
-  MT_REQUIRE((dgamma == nullptr) == (dbeta == nullptr), "layernorm bwd: dgamma and dbeta go together");
-  if (cols == 768)
-    return dispatch_ln_bwd<768, false>(dy, dy_dtype, x, x_dtype, nullptr, gamma, mean, rstd, residual, res_dtype, dx, dx_dtype, dx_bf16, dgamma, dbeta, rows, st);
-  if (cols == 3072)
-    return dispatch_ln_bwd<3072, false>(dy, dy_dtype, x, x_dtype, nullptr, gamma, mean, rstd, residual, res_dtype, dx, dx_dtype, dx_bf16, dgamma, dbeta, rows, st);
-  set_error("layernorm bwd: width %lld not supported (768, 3072)", (long long)cols);
-  return MT_E_UNSUPPORTED;
+  return layernorm_bwd(dy, dy_dtype, x, x_dtype, gamma, mean, rstd, residual, res_dtype, dx, dx_dtype, dx_bf16, dgamma,
+                       dbeta, rows, cols, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int mt_layernorm_bwd_ws(const void* dy, int dy_dtype, const void* x, int x_dtype, const float* gamma,
+                                   const float* mean, const float* rstd, const void* residual, int res_dtype, void* dx,
+                                   int dx_dtype, void* dx_bf16, float* dgamma, float* dbeta, int64_t rows, int64_t cols,
+                                   float* workspace, int64_t workspace_floats, void* stream) {
+  MT_REQUIRE(dgamma == nullptr || (workspace != nullptr && workspace_floats >= mt_colreduce_workspace_floats(cols)),
+             "layernorm bwd: workspace too small");
+  return layernorm_bwd(dy, dy_dtype, x, x_dtype, gamma, mean, rstd, residual, res_dtype, dx, dx_dtype, dx_bf16, dgamma,
+                       dbeta, rows, cols, dgamma != nullptr ? workspace : nullptr, (cudaStream_t)stream);
 }
 
 extern "C" int mt_gelu_ln_fwd(const void* h, int h_dtype, const float* hbias, const float* gamma, const float* beta,
@@ -873,29 +950,48 @@ extern "C" int mt_add_layernorm_fwd(const float* x, const void* a, int a_dtype, 
   return check_launch("add_ln_fwd_kernel");
 }
 
-extern "C" int mt_gated_residual_bwd(const float* dy, const float* a, const void* b, int b_dtype, const float* gate,
-                                     float* da, void* db, int db_dtype, float* dgate, float* dysum, int64_t rows,
-                                     int64_t cols, void* stream) {
+static int gated_residual_bwd(const float* dy, const float* a, const void* b, int b_dtype, const float* gate, float* da,
+                              void* db, int db_dtype, float* dgate, float* dysum, int64_t rows, int64_t cols, float* part,
+                              cudaStream_t st) {
   MT_REQUIRE(cols % 8 == 0 && cols / 8 <= 256, "gated_residual_bwd: cols must be a multiple of 8, at most 2048");
   MT_REQUIRE(b_dtype == db_dtype, "gated_residual_bwd: db must have the dtype of b");
   MT_REQUIRE(gate != nullptr && dgate != nullptr, "gated_residual_bwd: gate and dgate are required");
-  cudaStream_t st = (cudaStream_t)stream;
-  MT_CUDA(cudaMemsetAsync(dgate, 0, sizeof(float) * (size_t)cols, st));
-  if (dysum != nullptr) MT_CUDA(cudaMemsetAsync(dysum, 0, sizeof(float) * (size_t)cols, st));
+  if (part == nullptr || rows == 0) {
+    MT_CUDA(cudaMemsetAsync(dgate, 0, sizeof(float) * (size_t)cols, st));
+    if (dysum != nullptr) MT_CUDA(cudaMemsetAsync(dysum, 0, sizeof(float) * (size_t)cols, st));
+  }
   if (rows == 0) return 0;
   const int chunks = (int)(cols / 8);
   const int rpb = 768 / chunks;                  // >= 3 (chunks <= 256)
   const int threads = chunks * rpb;
   int grid = grid_for(rows, rpb);
   if (grid > kNumSMs) grid = kNumSMs;            // one 768-thread block per SM; bounds the number of reduce-add flushes
+  static_assert(kNumSMs <= kColReduceBlocks, "partials of the deterministic variant");
   const size_t smem = sizeof(float) * 8 * (size_t)chunks * (rpb - 1);
   MT_REQUIRE(((reinterpret_cast<uintptr_t>(dgate) | reinterpret_cast<uintptr_t>(dysum)) & 15) == 0,
              "gated_residual_bwd: dgate / dysum must be 16-byte aligned");
   if (b_dtype == MT_F32)
-    gated_residual_bwd_kernel<float><<<grid, threads, smem, st>>>(dy, a, (const float*)b, gate, da, (float*)db, dgate, dysum, rows, (int)cols);
+    gated_residual_bwd_kernel<float><<<grid, threads, smem, st>>>(dy, a, (const float*)b, gate, da, (float*)db, dgate, dysum, rows, (int)cols, part);
   else
-    gated_residual_bwd_kernel<__nv_bfloat16><<<grid, threads, smem, st>>>(dy, a, (const __nv_bfloat16*)b, gate, da, (__nv_bfloat16*)db, dgate, dysum, rows, (int)cols);
-  return check_launch("gated_residual_bwd_kernel");
+    gated_residual_bwd_kernel<__nv_bfloat16><<<grid, threads, smem, st>>>(dy, a, (const __nv_bfloat16*)b, gate, da, (__nv_bfloat16*)db, dgate, dysum, rows, (int)cols, part);
+  if (int rc = check_launch("gated_residual_bwd_kernel")) return rc;
+  return part != nullptr ? sum_partials(part, grid, (int)cols, dgate, dysum, st) : 0;
+}
+
+extern "C" int mt_gated_residual_bwd(const float* dy, const float* a, const void* b, int b_dtype, const float* gate,
+                                     float* da, void* db, int db_dtype, float* dgate, float* dysum, int64_t rows,
+                                     int64_t cols, void* stream) {
+  return gated_residual_bwd(dy, a, b, b_dtype, gate, da, db, db_dtype, dgate, dysum, rows, cols, nullptr,
+                            (cudaStream_t)stream);
+}
+
+extern "C" int mt_gated_residual_bwd_ws(const float* dy, const float* a, const void* b, int b_dtype, const float* gate,
+                                        float* da, void* db, int db_dtype, float* dgate, float* dysum, int64_t rows,
+                                        int64_t cols, float* workspace, int64_t workspace_floats, void* stream) {
+  MT_REQUIRE(workspace != nullptr && workspace_floats >= mt_colreduce_workspace_floats(cols),
+             "gated_residual_bwd: workspace too small");
+  return gated_residual_bwd(dy, a, b, b_dtype, gate, da, db, db_dtype, dgate, dysum, rows, cols, workspace,
+                            (cudaStream_t)stream);
 }
 
 extern "C" int mt_residual_bias_add(const float* x, const void* a, int a_dtype, const float* bias, float* y,
@@ -949,23 +1045,33 @@ extern "C" int mt_ffn_bwd_prep(const float* dy, const float* y, const float* x1,
   return check_launch("ffn_bwd_prep_kernel");
 }
 
-extern "C" int mt_colsum(const float* x, int64_t ld, float* out, int64_t rows, int64_t cols, void* stream) {
+static int colsum(const float* x, int64_t ld, float* out, int64_t rows, int64_t cols, float* part, cudaStream_t st) {
   MT_REQUIRE(x != nullptr && out != nullptr && rows >= 0, "colsum: NULL argument");
   MT_REQUIRE(cols > 0 && cols % 4 == 0 && cols <= 4096 && ld >= cols && ld % 4 == 0, "colsum: cols must be a multiple of 4, at most 4096");
-  MT_REQUIRE((((uintptr_t)x | (uintptr_t)out) & 15) == 0, "colsum: 16-byte alignment");
-  cudaStream_t st = (cudaStream_t)stream;
-  MT_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)cols, st));
+  MT_REQUIRE((((uintptr_t)x | (uintptr_t)out | (uintptr_t)part) & 15) == 0, "colsum: 16-byte alignment");
+  if (part == nullptr || rows == 0) MT_CUDA(cudaMemsetAsync(out, 0, sizeof(float) * (size_t)cols, st));
   if (rows == 0) return 0;
   const int quads = (int)(cols / 4);
   int row_lanes = 1024 / quads;
   if (row_lanes > 8) row_lanes = 8;
   if (row_lanes > rows) row_lanes = (int)rows;
   int64_t grid = (rows + (int64_t)row_lanes * 4 - 1) / ((int64_t)row_lanes * 4);   // >= 4 rows per lane
-  if (grid > 2 * kNumSMs) grid = 2 * kNumSMs;
+  if (grid > kColReduceBlocks) grid = kColReduceBlocks;
   if (grid < 1) grid = 1;
   const size_t smem = sizeof(float4) * (size_t)quads * (size_t)(row_lanes > 1 ? row_lanes - 1 : 1);
-  colsum_kernel<<<(unsigned)grid, quads * row_lanes, smem, st>>>(x, ld, out, rows, quads, row_lanes);
-  return check_launch("colsum_kernel");
+  colsum_kernel<<<(unsigned)grid, quads * row_lanes, smem, st>>>(x, ld, out, rows, quads, row_lanes, (float4*)part);
+  if (int rc = check_launch("colsum_kernel")) return rc;
+  return part != nullptr ? sum_partials(part, (int)grid, (int)cols, out, nullptr, st) : 0;
+}
+
+extern "C" int mt_colsum(const float* x, int64_t ld, float* out, int64_t rows, int64_t cols, void* stream) {
+  return colsum(x, ld, out, rows, cols, nullptr, (cudaStream_t)stream);
+}
+
+extern "C" int mt_colsum_ws(const float* x, int64_t ld, float* out, int64_t rows, int64_t cols, float* workspace,
+                            int64_t workspace_floats, void* stream) {
+  MT_REQUIRE(workspace != nullptr && workspace_floats >= mt_colreduce_workspace_floats(cols), "colsum: workspace too small");
+  return colsum(x, ld, out, rows, cols, workspace, (cudaStream_t)stream);
 }
 
 extern "C" int mt_layernorm_bwd_ffn_prep(const float* dy, const float* x, const float* gamma, const float* mean,

@@ -83,6 +83,16 @@ def _f32(t: torch.Tensor) -> torch.Tensor:
     return t if t.dtype == torch.float32 else t.float()
 
 
+def _deterministic() -> bool:
+    from . import config
+    return config.deterministic()
+
+
+def _colreduce_workspace(device, cols: int) -> torch.Tensor:
+    """Block partials of a deterministic column reduction (``mt_*_ws``); under graph capture from the graph's pool."""
+    return torch.empty(int(_lib.load().mt_colreduce_workspace_floats(cols)), device=device, dtype=torch.float32)
+
+
 # ---------------------------------------------------------------------------------------------------------------------
 # dilated-attention geometry
 # ---------------------------------------------------------------------------------------------------------------------
@@ -153,12 +163,22 @@ def layernorm_bwd(dy, x, gamma, mean, rstd, dx_dtype, residual=None, want_wgrad:
     dx = out if out is not None else torch.empty((rows, cols), device=x.device, dtype=dx_dtype)
     twin = torch.empty((rows, cols), device=x.device, dtype=torch.bfloat16) if bf16_twin else None
     dgamma = dbeta = None
+    lib = _lib.load()
+    args = (_p(dy), _dt(dy), _p(x), _dt(x), _p(gamma), _p(mean), _p(rstd), _p(residual),
+            _dt(residual) if residual is not None else 0, _p(dx), _dt(dx), _p(twin))
+    if want_wgrad and _deterministic():
+        dgb = torch.empty((2, cols), device=x.device, dtype=torch.float32)   # written, not accumulated
+        dgamma, dbeta = dgb[0], dgb[1]
+        ws = _colreduce_workspace(x.device, cols)
+        rc = lib.mt_layernorm_bwd_ws(*args, _p(dgamma), _p(dbeta), rows, cols, _p(ws), ws.numel(), _stream())
+        _check(rc, "mt_layernorm_bwd_ws", 2)
+        if twin is not None:
+            dx._mt_bf16 = twin
+        return dx, dgamma, dbeta
     if want_wgrad:
         dgb = torch.zeros((2, cols), device=x.device, dtype=torch.float32)   # one fill for both accumulators
         dgamma, dbeta = dgb[0], dgb[1]
-    rc = _lib.load().mt_layernorm_bwd(_p(dy), _dt(dy), _p(x), _dt(x), _p(gamma), _p(mean), _p(rstd), _p(residual),
-                                      _dt(residual) if residual is not None else 0, _p(dx), _dt(dx), _p(twin),
-                                      _p(dgamma), _p(dbeta), rows, cols, _stream())
+    rc = lib.mt_layernorm_bwd(*args, _p(dgamma), _p(dbeta), rows, cols, _stream())
     _check(rc, "mt_layernorm_bwd")
     if twin is not None:
         dx._mt_bf16 = twin
@@ -284,15 +304,28 @@ def dilated_merge_ln_bwd(geom: Geometry, dy, o_br, lse_br, gamma, mean, rstd):
     return dattn, delta_br
 
 
+def dilated_bwd_impl(impl: int) -> int:
+    """The backward kernel that runs for the requested ``impl``: in deterministic mode the tcgen05 backward (1, 2) runs
+    as impl 4, the deterministic one; the SIMT backward (0) has no deterministic variant and raises there."""
+    from . import config
+    if impl == 0:
+        config.check_deterministic("the SIMT dilated-attention backward (fp32 mode, or attn_impl simt)")
+    elif impl in (1, 2) and config.deterministic():
+        return config.DETERMINISTIC_BWD_IMPL
+    return impl
+
+
 def dilated_attn_bwd(geom: Geometry, qkv, dattn, lse, delta_br, impl: int):
     """dattn [n_alloc, E] (rows >= N zero), merged lse [N, H], per-branch delta -> dqkv fp32 [N, 3E]."""
     N, E = geom.n_tokens, geom.heads * geom.head_dim
     assert dattn.shape[0] == geom.n_alloc, "dattn must have n_alloc rows (zero tail), see dilated_merge_ln_bwd"
+    impl = dilated_bwd_impl(impl)
     dqkv = torch.empty((geom.n_alloc, 3 * E), device=qkv.device, dtype=torch.float32)  # rows >= N: reduce scratch
     with _timed("dilated_attn_bwd"):
         rc = _lib.load().mt_dilated_attn_bwd(geom.ref(), _p(qkv), qkv.stride(0), qkv.shape[0], _p(dattn), _p(lse),
                                              _p(delta_br), _dt(qkv), _p(dqkv), impl, _stream())
-    _check(rc, "mt_dilated_attn_bwd", 2)
+    # memset + kernel; the deterministic backward (impl 4) launches a dQ and a dK / dV kernel per branch
+    _check(rc, "mt_dilated_attn_bwd", 1 + (2 * len(geom.ratios) if impl == 4 else 1))
     return dqkv[:N]
 
 
@@ -340,6 +373,11 @@ def cross_attn_bwd(q, k, v, o, d_o, lse, heads: int, impl: Optional[int] = None,
         _rows_ok(t)
     assert k.stride(0) == v.stride(0) and o.stride(0) == d_o.stride(0)
     impl = cross_impl(q) if impl is None else impl
+    det = _deterministic()
+    if det and impl == 0:
+        from . import config
+        config.check_deterministic("the SIMT cross-attention backward (fp32 mode, or cross_tc off)")
+        det = False   # warn_only: the warning is all torch's flag asks for
     dq = torch.empty((lq, e), device=q.device, dtype=torch.float32)
     if packed_kv:
         dkv = torch.empty((lk, 2 * e), device=q.device, dtype=torch.float32)
@@ -347,9 +385,18 @@ def cross_attn_bwd(q, k, v, o, d_o, lse, heads: int, impl: Optional[int] = None,
     else:
         dk = torch.empty((lk, e), device=q.device, dtype=torch.float32)
         dv = torch.empty((lk, e), device=q.device, dtype=torch.float32)
-    rc = _lib.load().mt_cross_attn_bwd(_ptr(q), q.stride(0), _ptr(k), _ptr(v), k.stride(0), _ptr(o), _ptr(d_o), o.stride(0),
-                                       _p(lse), _dt(q), _ptr(dq), dq.stride(0), _ptr(dk), _ptr(dv), dk.stride(0), lq, lk,
-                                       heads, e // heads, impl, _stream())
+    lib = _lib.load()
+    args = (_ptr(q), q.stride(0), _ptr(k), _ptr(v), k.stride(0), _ptr(o), _ptr(d_o), o.stride(0), _p(lse), _dt(q), _ptr(dq),
+            dq.stride(0), _ptr(dk), _ptr(dv), dk.stride(0), lq, lk, heads, e // heads)
+    if det:
+        # split loops store partials that a second pass sums in split order (no atomics); workspace from the graph's
+        # pool under capture
+        nws = int(lib.mt_cross_attn_bwd_workspace_floats(lq, lk, heads, e // heads, _dt(q), impl))
+        ws = torch.empty(max(nws, 4), device=q.device, dtype=torch.float32)
+        rc = lib.mt_cross_attn_bwd_ws(*args, _p(ws), nws, impl, _stream())
+        _check(rc, "mt_cross_attn_bwd_ws", 2 if nws else 1)
+        return dq, dk, dv
+    rc = lib.mt_cross_attn_bwd(*args, impl, _stream())
     _check(rc, "mt_cross_attn_bwd", 5)
     return dq, dk, dv
 
@@ -435,6 +482,12 @@ def colsum(x: torch.Tensor) -> torch.Tensor:
             and x.stride(0) % 4 == 0 and x.data_ptr() % 16 == 0 and rows >= 1024):
         return x.sum(0)            # short inputs (the 66 modal tokens): one library launch instead of memset + kernel
     out = torch.empty(cols, device=x.device, dtype=torch.float32)
+    if _deterministic():
+        ws = _colreduce_workspace(x.device, cols)
+        rc = _lib.load().mt_colsum_ws(ctypes.c_void_p(x.data_ptr()), x.stride(0), _p(out), rows, cols, _p(ws), ws.numel(),
+                                      _stream())
+        _check(rc, "mt_colsum_ws", 2)
+        return out
     rc = _lib.load().mt_colsum(ctypes.c_void_p(x.data_ptr()), x.stride(0), _p(out), rows, cols, _stream())
     _check(rc, "mt_colsum")
     return out
@@ -547,9 +600,14 @@ def gated_residual_bwd(dy, a, b, g32, out=None, want_dysum: bool = False):
     db = torch.empty_like(b)
     dgate = torch.empty(cols, device=a.device, dtype=torch.float32)
     dysum = torch.empty(cols, device=a.device, dtype=torch.float32) if want_dysum else None
-    rc = _lib.load().mt_gated_residual_bwd(_p(dy), _p(a), _p(b), _dt(b), _p(g32), _p(da), _p(db), _dt(db), _p(dgate),
-                                           _p(dysum), rows, cols, _stream())
-    _check(rc, "mt_gated_residual_bwd")
+    args = (_p(dy), _p(a), _p(b), _dt(b), _p(g32), _p(da), _p(db), _dt(db), _p(dgate), _p(dysum), rows, cols)
+    if _deterministic():
+        ws = _colreduce_workspace(a.device, cols)
+        rc = _lib.load().mt_gated_residual_bwd_ws(*args, _p(ws), ws.numel(), _stream())
+        _check(rc, "mt_gated_residual_bwd_ws", 2)
+    else:
+        rc = _lib.load().mt_gated_residual_bwd(*args, _stream())
+        _check(rc, "mt_gated_residual_bwd")
     return (da, db, dgate, dysum) if want_dysum else (da, db, dgate)
 
 

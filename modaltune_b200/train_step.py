@@ -297,6 +297,12 @@ class GraphedStep:
         self._warmup, self._pool = warmup, pool
         self._capture()
 
+    def _capture_signature(self):
+        """What the captured kernels depend on besides the inputs: the deterministic switch (a graph captured with the
+        fast backward must never replay as deterministic, nor the other way round) and the frozen weights."""
+        from . import config
+        return config.deterministic(), self._frozen_signature()
+
     def _frozen_signature(self):
         """Identity + version of every frozen parameter the captured kernels read through derived copies
         (``ops.FrozenLayerWeights``): a ``load_state_dict`` / in-place edit after capture changes it."""
@@ -325,7 +331,7 @@ class GraphedStep:
                 flat.densify()     # gradients in parameter layout: the optimizer's multi-tensor path
         # views of the captured flat buffer, handed back to ``p.grad`` after every replay
         self._grad_views = [p.grad for p in flat.params]
-        self._signature = self._frozen_signature()
+        self._signature = self._capture_signature()
 
     @property
     def grads(self) -> torch.Tensor:
@@ -388,8 +394,9 @@ class GraphedStep:
         """``reduce``: all-reduce the flat gradients over the data-parallel ranks after the replay (one slide per rank and
         step).  ``GraphCache`` passes False: ranks step through different numbers of slides and exchange the accumulated
         gradients once."""
-        if self._frozen_signature() != self._signature:
-            # the graph holds pointers to bf16 copies derived from the old frozen weights: capture again
+        if self._capture_signature() != self._signature:
+            # the graph holds pointers to bf16 copies derived from the old frozen weights, or was captured with the
+            # other setting of the deterministic switch: capture again
             self._capture()
         if packed is not None:
             self.load(packed)
