@@ -253,6 +253,17 @@ int mt_cross_attn_bwd_ws(const void* q, int64_t ldq, const void* k, const void* 
                          float* dk_f32, float* dv_f32, int64_t lddkv, int64_t lq, int64_t lk, int heads, int head_dim,
                          float* workspace, int64_t workspace_floats, int impl, void* stream);
 int64_t mt_cross_attn_bwd_workspace_floats(int64_t lq, int64_t lk, int heads, int head_dim, int dtype, int impl);
+/* Head-averaged attention probabilities of a mt_cross_attn_fwd call:  p[i, j] = (1/heads) sum_h exp(q_i^h . k_j^h / 4
+ * - lse[i, h]), p [Lq, Lk] f32 with row stride ldp >= Lk.
+ * replaces: the attn_weights output (need_weights=True, average_attn_weights=True) of the nn.MultiheadAttention calls of
+ * SelfAttentionLayer.forward_pre and CrossAttentionLayer.forward_pre (models/vitadapter/adapter_modules.py:72,87,198,225),
+ * which a forward hook on `self_attn` / `multihead_attn` receives.
+ * q, k, lse and impl as passed to (and lse as returned by) mt_cross_attn_fwd; k may be any column slice with row stride
+ * ldk (the k half of the [Lk, 2E'] k|v buffer, or of a wider shared projection).  The scores are recomputed with the
+ * forward's arithmetic (impl 1: TF32 operands, q scaled by log2(e)/4 before rounding), so each row sums to 1 up to
+ * rounding.  Every element of p is written exactly once (no atomics): the output is bitwise reproducible. */
+int mt_cross_attn_probs(const void* q, int64_t ldq, const void* k, int64_t ldk, int dtype, const float* lse, float* p,
+                        int64_t ldp, int64_t lq, int64_t lk, int heads, int head_dim, int impl, void* stream);
 
 /* ---- small fused element-wise pieces ------------------------------------------------------------------------------
  * y[r, c] = a[r, c] + gate[c] * (a[r, c] + b[r, c])      Injector tail `query + gamma * attn` (adapter_modules.py:362)

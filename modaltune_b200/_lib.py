@@ -81,6 +81,7 @@ SIGNATURES = {
     "mt_cross_attn_bwd_ws": (c_int, [_P, _I64, _P, _P, _I64, _P, _P, _I64, _P, c_int, _P, _I64, _P, _P, _I64, _I64, _I64,
                                      c_int, c_int, _P, _I64, c_int, _P]),
     "mt_cross_attn_bwd_workspace_floats": (_I64, [_I64, _I64, c_int, c_int, c_int, c_int]),
+    "mt_cross_attn_probs": (c_int, [_P, _I64, _P, _I64, c_int, _P, _P, _I64, _I64, _I64, c_int, c_int, c_int, _P]),
     "mt_gated_residual": (c_int, [_P, _P, c_int, _P, _P, _I64, _I64, _P]),
     "mt_gated_residual_bwd": (c_int, [_P, _P, _P, c_int, _P, _P, _P, c_int, _P, _P, _I64, _I64, _P]),
     "mt_gated_residual_bwd_ws": (c_int, [_P, _P, _P, c_int, _P, _P, _P, c_int, _P, _P, _I64, _I64, _P, _I64, _P]),

@@ -9,11 +9,13 @@ What runs where: LayerNorm (+ fused positional add), the 12-head x 16 softmax(QK
 Injector's many-queries/few-keys shape, split-K + LSE combine for the Extractor's few-queries/many-keys shape) and the
 gated residual tail are hand-written kernels (``ops.LayerNormFn`` / ``CrossAttnFn`` / ``GatedResidualFn``); the skinny
 trainable projections (768<->192) are cuBLAS GEMMs through autograd.  The reference's ``nn.MultiheadAttention`` call
-materialises [12, Lq, Lk] probabilities and their head average (discarded, :225-229); nothing of that size exists here.
+materialises [12, Lq, Lk] probabilities and their head average (discarded, :225-229); nothing of that size exists here,
+except the [Lq, Lk] head average when a forward hook on the attention module asks for it (``MultiheadAttention``).
 """
 from __future__ import annotations
 
-from typing import Optional
+import contextlib
+from typing import List, Optional
 
 import torch
 import torch.nn as nn
@@ -56,20 +58,88 @@ def _lin(x, w, b):
     return F.linear(x, w, b)
 
 
-def _mha_core(mha: nn.MultiheadAttention, query, key, value):
+def _mha_core(mha: nn.MultiheadAttention, query, key, value, need_weights: bool = False):
     """The arithmetic of ``nn.MultiheadAttention(E', heads, kdim=vdim=768, batch_first)`` with separate q/k/v weights
-    on 2-D operands: in-projections, softmax(QK^T/sqrt(hd))V (kernel), out-projection."""
+    on 2-D operands: in-projections, softmax(QK^T/sqrt(hd))V (kernel), out-projection.  ``need_weights``: also return the
+    head-averaged probabilities [Lq, Lk] fp32 (detached), recomputed by ``ops.cross_attn_probs`` from the forward's q, k
+    and lse."""
     e = mha.embed_dim
     b = mha.in_proj_bias
     q = _lin(query, mha.q_proj_weight, b[:e])
     if key is value:
         kv = _lin(key, torch.cat([mha.k_proj_weight, mha.v_proj_weight], 0), b[e:])
-        o = ops.cross_attention_kv(q, kv, mha.num_heads)   # k | v read in place, gradient returned as one tensor
+        # k | v read in place, gradient returned as one tensor
+        o, lse = ops.cross_attention_kv(q, kv, mha.num_heads, return_lse=True)
+        k = kv[:, :e]
     else:
         k = _lin(key, mha.k_proj_weight, b[e:2 * e])
         v = _lin(value, mha.v_proj_weight, b[2 * e:])
-        o = ops.cross_attention(q, k, v, mha.num_heads)
-    return _lin(o, mha.out_proj.weight, mha.out_proj.bias)
+        o, lse = ops.cross_attention(q, k, v, mha.num_heads, return_lse=True)
+    out = _lin(o, mha.out_proj.weight, mha.out_proj.bias)
+    if not need_weights:
+        return out
+    with torch.no_grad():
+        return out, ops.cross_attn_probs(q.detach(), k.detach(), lse, mha.num_heads)
+
+
+# tensors returned to forward hooks while a task pass runs on a side stream (``recording_outputs``)
+_side_outputs: Optional[List[torch.Tensor]] = None
+
+
+@contextlib.contextmanager
+def recording_outputs(sink: List[torch.Tensor]):
+    """Inside the block, every tensor a ``MultiheadAttention`` forward returns is appended to ``sink``: the caller that
+    ran the block on a side stream makes them safe to use on its own stream (``record_stream``)."""
+    global _side_outputs
+    old, _side_outputs = _side_outputs, sink
+    try:
+        yield
+    finally:
+        _side_outputs = old
+
+
+class MultiheadAttention(nn.MultiheadAttention):
+    """``nn.MultiheadAttention`` (same parameters, names and state dict) whose ``forward`` runs the adapter's kernels.
+
+    The adapter layers call ``_mha_core`` directly; they go through this module (``nn.Module.__call__``, so torch's hook
+    semantics apply, including a hook that replaces the output) only when it has forward hooks or forward pre-hooks.
+    The hooks then receive what the reference's ``need_weights=True`` call returns: ``(attn_output [1, Lq, E'],
+    attn_weights [1, Lq, Lk])``, the weights averaged over the heads, fp32 and detached (no autograd history).  Global
+    hooks (``nn.modules.module.register_module_forward_hook``) do not reroute the layers."""
+
+    def forward(self, query, key, value, key_padding_mask=None, need_weights=True, attn_mask=None,
+                average_attn_weights=True, is_causal=False):
+        if key_padding_mask is not None or attn_mask is not None or is_causal:
+            raise NotImplementedError("modaltune_b200 MultiheadAttention: key_padding_mask, attn_mask and is_causal are "
+                                      "not supported (the ModalTune adapter never uses them)")
+        if need_weights and not average_attn_weights:
+            raise NotImplementedError("modaltune_b200 MultiheadAttention: per-head weights (average_attn_weights=False) "
+                                      "are not supported; only the head average is computed")
+        assert self.batch_first, "modaltune_b200 MultiheadAttention takes batch-first [1, L, E] inputs"
+        k = _rows(key)
+        res = _mha_core(self, _rows(query), k, k if value is key else _rows(value), need_weights)
+        out, w = (res[0].unsqueeze(0), res[1].unsqueeze(0)) if need_weights else (res.unsqueeze(0), None)
+        if _side_outputs is not None:
+            _side_outputs.extend(t for t in (out, w) if t is not None)
+        return out, w
+
+
+def _hooked(m: nn.Module) -> bool:
+    return bool(m._forward_hooks or m._forward_pre_hooks)
+
+
+def hooked_attention(modules) -> List[str]:
+    """Names of the adapter attention modules among ``modules`` ((name, module) pairs) that have forward hooks."""
+    return [n for n, m in modules if isinstance(m, MultiheadAttention) and _hooked(m)]
+
+
+def _attend(mha: nn.MultiheadAttention, query, key, value):
+    """``_mha_core`` on 2-D operands, or the module call with [1, L, E] views when ``mha`` is hooked."""
+    if not _hooked(mha):
+        return _mha_core(mha, query, key, value)
+    k = key.unsqueeze(0)
+    out = mha(query=query.unsqueeze(0), key=k, value=k if value is key else value.unsqueeze(0))
+    return _rows(out[0])
 
 
 def _rows(t: torch.Tensor) -> torch.Tensor:
@@ -97,8 +167,8 @@ class SelfAttentionLayer(nn.Module):
             embed_model = int(d_model * cffn_ratio)
             self.q_proj = nn.Linear(d_model, embed_model)
             self.output_proj = nn.Linear(embed_model, d_model)
-        self.self_attn = nn.MultiheadAttention(embed_model, nheads, dropout=dropout, batch_first=True, kdim=d_model,
-                                               vdim=d_model)
+        self.self_attn = MultiheadAttention(embed_model, nheads, dropout=dropout, batch_first=True, kdim=d_model,
+                                            vdim=d_model)
         self.norm = nn.LayerNorm(d_model)
         self.dropout = nn.Dropout(dropout)
         self.normalize_before = normalize_before
@@ -114,7 +184,7 @@ class SelfAttentionLayer(nn.Module):
         t2 = ops.layer_norm(t, self.norm.weight, self.norm.bias)
         qk = t2 if query_pos is None else t2 + _pos_rows(query_pos, t.shape[0]).to(t2.dtype)
         query = _lin(qk, self.q_proj.weight, self.q_proj.bias) if self.with_cffn else qk
-        a = _mha_core(self.self_attn, query, qk, t2)
+        a = _attend(self.self_attn, query, qk, t2)
         if self.with_cffn:
             a = _lin(a, self.output_proj.weight, self.output_proj.bias)
         return (t + self.dropout(a)).unsqueeze(0)
@@ -134,8 +204,8 @@ class CrossAttentionLayer(nn.Module):
             embed_model = int(d_model * cffn_ratio)
             self.q_proj = nn.Linear(d_model, embed_model)
             self.output_proj = nn.Linear(embed_model, d_model)
-        self.multihead_attn = nn.MultiheadAttention(embed_model, nheads, dropout=dropout, batch_first=True,
-                                                    kdim=d_model, vdim=d_model)
+        self.multihead_attn = MultiheadAttention(embed_model, nheads, dropout=dropout, batch_first=True,
+                                                 kdim=d_model, vdim=d_model)
         if normalize_before:
             self.norm_kq = nn.LayerNorm(d_model)
         self.norm = nn.LayerNorm(d_model)
@@ -158,7 +228,7 @@ class CrossAttentionLayer(nn.Module):
         mem = ops.layer_norm(memory, self.norm_kq.weight, self.norm_kq.bias,
                              add=_pos_rows(pos, memory.shape[0] - mem_row0), row0=mem_row0)
         query = _lin(t2, self.q_proj.weight, self.q_proj.bias) if self.with_cffn else t2
-        a = _mha_core(self.multihead_attn, query, mem, mem)
+        a = _attend(self.multihead_attn, query, mem, mem)
         if self.with_cffn:
             a = _lin(a, self.output_proj.weight, self.output_proj.bias)
         return self.dropout(a)
@@ -292,7 +362,7 @@ class Injector(nn.Module):
 
     def _can_fuse(self):
         cl = self.attn
-        return (config.flag("injector_fused") and cl.normalize_before
+        return (config.flag("injector_fused") and cl.normalize_before and not _hooked(cl.multihead_attn)
                 and not (self.training and (cl.dropout.p > 0.0 or cl.multihead_attn.dropout > 0.0)))
 
     def forward_full(self, xfull, feat, pos=None):
@@ -343,10 +413,12 @@ class InteractionBlockWithCls_LongNetViT(InteractionBlockWithCls):
         for idx, blk in enumerate(blocks):
             xfull, _ = blk(xfull, incremental_state=(incremental_state[idx] if incremental_state is not None else None),
                            **layer_configs)
-        if self.extra_extractors is not None and config.shared_extractor_kv():
+        exts = [self.extractor, *(self.extra_extractors or ())]
+        if (self.extra_extractors is not None and config.shared_extractor_kv()
+                and not any(_hooked(e.attn.multihead_attn) for e in exts)):
             # the three extractors of the last block read the same slide tokens: one normalisation pass and one GEMM
-            # for all their k | v projections (ops.SharedKVProjectFn), each then attends on its column slice
-            exts = [self.extractor, *self.extra_extractors]
+            # for all their k | v projections (ops.SharedKVProjectFn), each then attends on its column slice.  A hooked
+            # extractor needs its own attention call: then every extractor of the block projects for itself
             wb = [e.kv_weights() for e in exts]
             kv_all = ops.shared_kv_project(_rows(xfull), torch.cat([w for w, _ in wb], 0), torch.cat([b for _, b in wb], 0), 1)
             for e, kv in zip(exts, torch.split(kv_all, kv_all.shape[1] // len(exts), dim=1)):

@@ -770,6 +770,126 @@ __global__ void __launch_bounds__(256) cross_split_sum_kernel(const float* __res
   out[r * ld_out + c] = acc;
 }
 
+// ---------------------------------------------------------------------------------------------------------------------
+// Head-averaged attention probabilities P[i, j] = (1/H) sum_h exp(s_ij^h - lse_ih): nn.MultiheadAttention's
+// need_weights=True output, for the forward hooks of the adapter's attention modules.  Both kernels recompute the scores
+// from the SAME operands with the SAME arithmetic as the forward of their impl (bitwise the same s) and take the lse that
+// forward returned, so a row sums to 1 against the probabilities the forward actually used.  Every output element is
+// written once by one thread, heads summed in index order in registers: no atomics, bitwise reproducible.
+// ---------------------------------------------------------------------------------------------------------------------
+static constexpr int PQ = 16;   // queries per CTA of the SIMT kernel (one thread per key, XT keys per CTA)
+
+// SIMT (impl 0): thread = one key, loops over PQ staged queries per head.  dot16(k, q / 4) forms the products and sums of
+// the forward's dot16(q / 4, k) in the same order (fma is commutative), so s is the forward's s bit for bit.
+template <typename T>
+__global__ void __launch_bounds__(XT) cross_probs_kernel(const T* __restrict__ q, int64_t ldq, const T* __restrict__ k,
+                                                         int64_t ldk, const float* __restrict__ lse, float* __restrict__ p,
+                                                         int64_t ldp, int64_t lq, int64_t lk, int heads) {
+  __shared__ __align__(16) float Qs[PQ * HD];
+  __shared__ float Ls[PQ];
+  const int64_t kj = (int64_t)blockIdx.x * XT + threadIdx.x, q0 = (int64_t)blockIdx.y * PQ;
+  const bool live = kj < lk;
+  float acc[PQ];
+#pragma unroll
+  for (int i = 0; i < PQ; ++i) acc[i] = 0.f;
+  for (int h = 0; h < heads; ++h) {
+    __syncthreads();
+    if (threadIdx.x < PQ) {
+      const int64_t qi = q0 + threadIdx.x;
+      float a[HD];
+      if (qi < lq) load16(q + qi * ldq + h * HD, a);
+      else
+#pragma unroll
+        for (int e = 0; e < HD; ++e) a[e] = 0.f;
+#pragma unroll
+      for (int e = 0; e < HD; ++e) Qs[threadIdx.x * HD + e] = a[e] * 0.25f;   // 1/sqrt(16), as the forward's to_pairs
+      Ls[threadIdx.x] = qi < lq ? lse[qi * heads + h] : 0.f;
+    }
+    __syncthreads();
+    float kv[HD];
+    if (live) load16(k + kj * ldk + h * HD, kv);
+    else
+#pragma unroll
+      for (int e = 0; e < HD; ++e) kv[e] = 0.f;
+    float2 k2[HD / 2];
+    to_pairs(kv, 1.f, k2);
+#pragma unroll
+    for (int i = 0; i < PQ; ++i) acc[i] += expf(dot16(k2, Qs + i * HD) - Ls[i]);
+  }
+  if (!live) return;
+  const float inv = 1.f / heads;
+#pragma unroll
+  for (int i = 0; i < PQ; ++i)
+    if (q0 + i < lq) p[(q0 + i) * ldp + kj] = acc[i] * inv;
+}
+
+// Tensor cores (impl 1, f32 tensors): warp = 16 queries, CTA = those warps x one chunk of TC keys (grid.x), heads looped
+// two at a time (stage2_tf32 stages head h into Ka and head h + 1 into Kb).  q is scaled by 0.25 log2e BEFORE the TF32
+// rounding and the score MMAs are the forward's mma_rows on the same fragments: P = ex2(s - lse log2e) is the forward's
+// probability.  The nine 16 x 8 accumulator tiles of the head sum stay in registers.
+__global__ void __launch_bounds__(256) cross_probs_tc_kernel(const float* __restrict__ q, int64_t ldq,
+                                                             const float* __restrict__ k, int64_t ldk,
+                                                             const float* __restrict__ lse, float* __restrict__ p,
+                                                             int64_t ldp, int64_t lq, int64_t lk, int heads) {
+  __shared__ __align__(16) uint32_t Ka[TC * TS], Kb[TC * TS];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
+  const int64_t r_lo = ((int64_t)blockIdx.y * (blockDim.x >> 5) + warp) * 16 + g, r_hi = r_lo + 8;
+  const int64_t k0 = (int64_t)blockIdx.x * TC;
+  const int cnt = (int)min((int64_t)TC, lk - k0), nt = (cnt + 7) >> 3;
+  float acc[TNT][4] = {};
+  for (int h0 = 0; h0 < heads; h0 += 2) {
+    const int npair = h0 + 1 < heads ? 2 : 1;
+    float qraw[2][2][4], L[2][2];
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {   // row operands of both heads in flight before the staging barrier
+      const int h = u < npair ? h0 + u : h0;
+      load_a_raw(qraw[u], q, ldq, h, r_lo, lq, t);
+      L[u][0] = r_lo < lq ? lse[r_lo * heads + h] : 0.f;
+      L[u][1] = r_hi < lq ? lse[r_hi * heads + h] : 0.f;
+    }
+    __syncthreads();
+    stage2_tf32(Ka, Kb, k, k + (npair - 1) * HD, ldk, h0, k0, lk);
+    __syncthreads();
+#pragma unroll
+    for (int u = 0; u < 2; ++u) {
+      if (u >= npair) break;
+      uint32_t qa[2][4];
+      cvt_a_frag(qa, qraw[u], 0.25f * kLog2e);
+      const float l_lo = L[u][0] * kLog2e, l_hi = L[u][1] * kLog2e;
+#pragma unroll
+      for (int j = 0; j < TNT; ++j) {
+        if (j < nt) {
+          float s[4] = {};
+          mma_rows(s, qa, u ? Kb : Ka, j, g, t);
+          acc[j][0] += ex2(s[0] - l_lo);
+          acc[j][1] += ex2(s[1] - l_lo);
+          acc[j][2] += ex2(s[2] - l_hi);
+          acc[j][3] += ex2(s[3] - l_hi);
+        }
+      }
+    }
+  }
+  const float inv = 1.f / heads;
+  const bool vec = (ldp & 1) == 0 && (reinterpret_cast<uintptr_t>(p) & 7) == 0;   // k0 and the column 2t are even
+#pragma unroll
+  for (int half = 0; half < 2; ++half) {
+    const int64_t r = half ? r_hi : r_lo;
+    if (r >= lq) continue;
+    float* row = p + r * ldp + k0;
+#pragma unroll
+    for (int j = 0; j < TNT; ++j) {
+      const int c = 8 * j + 2 * t;
+      const float v0 = acc[j][2 * half] * inv, v1 = acc[j][2 * half + 1] * inv;
+      if (vec && c + 1 < cnt) {
+        *reinterpret_cast<float2*>(row + c) = make_float2(v0, v1);
+      } else {
+        if (c < cnt) row[c] = v0;
+        if (c + 1 < cnt) row[c + 1] = v1;
+      }
+    }
+  }
+}
+
 // rows_parallel rows spread over CTAs of `rows_per_cta`, the other side looped in chunks of `chunk`: how many loop splits?
 static int pick_splits(int64_t rows_parallel, int64_t loop_len, int heads, int rows_per_cta, int chunk, bool tc) {
   const int64_t ctas = ((rows_parallel + rows_per_cta - 1) / rows_per_cta) * heads;
@@ -848,6 +968,35 @@ extern "C" int mt_cross_attn_fwd(const void* q, int64_t ldq, const void* k, cons
     return MT_E_BADARG;
   }
   return check_launch("cross_fwd_kernel");
+}
+
+extern "C" int mt_cross_attn_probs(const void* q, int64_t ldq, const void* k, int64_t ldk, int dtype, const float* lse,
+                                   float* p, int64_t ldp, int64_t lq, int64_t lk, int heads, int head_dim, int impl,
+                                   void* stream) {
+  MT_REQUIRE(head_dim == HD, "cross_attn_probs: head_dim must be 16 (got %d)", head_dim);
+  MT_REQUIRE(lq > 0 && lk > 0 && heads > 0, "cross_attn_probs: bad sizes");
+  MT_REQUIRE(impl == 0 || impl == 1, "cross_attn_probs: impl must be 0 (SIMT fp32) or 1 (TF32 tensor cores)");
+  MT_REQUIRE(dtype == MT_F32 || dtype == MT_BF16, "cross_attn_probs: bad dtype %d", dtype);
+  const int64_t e = (int64_t)heads * HD;
+  MT_REQUIRE(ldq >= e && ldk >= e && ((ldq | ldk) & 7) == 0 && ldp >= lk, "cross_attn_probs: bad row strides");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (use_tc(impl, dtype)) {
+    const int warps = tc_warps(lq);
+    const int64_t gy = (lq + 16 * warps - 1) / (16 * warps), gx = (lk + TC - 1) / TC;
+    MT_REQUIRE(gy <= 65535 && gx < (1ll << 31), "cross_attn_probs: too many queries");
+    cross_probs_tc_kernel<<<dim3((unsigned)gx, (unsigned)gy), 32 * warps, 0, st>>>((const float*)q, ldq, (const float*)k,
+                                                                                 ldk, lse, p, ldp, lq, lk, heads);
+    return check_launch("cross_probs_tc_kernel");
+  }
+  const int64_t gy = (lq + PQ - 1) / PQ, gx = (lk + XT - 1) / XT;
+  MT_REQUIRE(gy <= 65535 && gx < (1ll << 31), "cross_attn_probs: too many queries");
+  const dim3 grid((unsigned)gx, (unsigned)gy);
+  if (dtype == MT_F32)
+    cross_probs_kernel<float><<<grid, XT, 0, st>>>((const float*)q, ldq, (const float*)k, ldk, lse, p, ldp, lq, lk, heads);
+  else
+    cross_probs_kernel<__nv_bfloat16><<<grid, XT, 0, st>>>((const __nv_bfloat16*)q, ldq, (const __nv_bfloat16*)k, ldk, lse,
+                                                           p, ldp, lq, lk, heads);
+  return check_launch("cross_probs_kernel");
 }
 
 // Plans of the two roles of the backward: tensor-core path: both roles of the one backward kernel run with the same CTA size

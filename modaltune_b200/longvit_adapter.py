@@ -16,7 +16,7 @@ import torch.nn.functional as F
 
 from . import config
 from .adapter_modules import (CrossAttentionLayer, Identity_mod, InteractionBlockWithCls_LongNetViT,
-                              SelfAttentionLayer)
+                              SelfAttentionLayer, recording_outputs)
 from .gene_encoder import GeneEncoder_Group
 from .slide_encoder import LongNetViT
 
@@ -180,6 +180,7 @@ class LongNetGeneAdapter(LongNetViT):
         cur = torch.cuda.current_stream()
         streams = self._task_streams(len(task_tokens) - 1)
         outs = [None] * len(task_tokens)
+        hook_outputs = []   # what forward hooks on the attention modules received on the side streams
         gene_inputs = list(genes.values()) if isinstance(genes, dict) else list(genes)
         for k, t in enumerate(task_tokens):
             if k == 0:
@@ -193,12 +194,14 @@ class LongNetGeneAdapter(LongNetViT):
             for tns in (emb, gene, clinical, t, *(gene_inputs if gene is None else ())):
                 if torch.is_tensor(tns) and tns.is_cuda:
                     tns.record_stream(st)
-            with torch.cuda.stream(st):
+            with torch.cuda.stream(st), recording_outputs(hook_outputs):
                 outs[k] = one_pass(t, k)
         outs[0] = one_pass(task_tokens[0], 0)
         for k in range(1, len(task_tokens)):
             cur.wait_stream(streams[k - 1])
             outs[k].record_stream(cur)   # allocated on the side stream, read by the cat below on the calling stream
+        for tns in hook_outputs:         # and these by the hook's owner after we return
+            tns.record_stream(cur)
         return torch.cat(outs, 0)
 
     def join_pass_streams(self):

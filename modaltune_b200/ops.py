@@ -364,6 +364,24 @@ def cross_attn_fwd(q, k, v, heads: int, impl: Optional[int] = None):
     return o, lse
 
 
+def cross_attn_probs(q, k, lse, heads: int, impl: Optional[int] = None):
+    """Head-averaged attention probabilities [Lq, Lk] fp32 of the ``cross_attn_fwd`` call that took ``q``, ``k`` (row-
+    strided views allowed) and returned ``lse``: nn.MultiheadAttention's ``need_weights=True`` output.  Pass the same
+    ``impl`` as that forward (default: the same selection)."""
+    lq, e = q.shape
+    lk = k.shape[0]
+    for t in (q, k):
+        _rows_ok(t)
+    assert k.dtype == q.dtype and lse.dtype == torch.float32 and lse.shape == (lq, heads) and lse.is_contiguous()
+    impl = cross_impl(q) if impl is None else impl
+    p = torch.empty((lq, lk), device=q.device, dtype=torch.float32)
+    with _timed("cross_attn_probs"):
+        rc = _lib.load().mt_cross_attn_probs(_ptr(q), q.stride(0), _ptr(k), k.stride(0), _dt(q), _p(lse), _p(p),
+                                             p.stride(0), lq, lk, heads, e // heads, impl, _stream())
+    _check(rc, "mt_cross_attn_probs")
+    return p
+
+
 def cross_attn_bwd(q, k, v, o, d_o, lse, heads: int, impl: Optional[int] = None, packed_kv: bool = False):
     """-> dq [Lq, E'], dk, dv [Lk, E'] fp32.  ``packed_kv``: dk / dv are the two halves of ONE [Lk, 2E'] buffer (returned
     as views), the layout the gradient of a fused k|v projection wants."""
@@ -549,7 +567,7 @@ class CrossAttnFn(torch.autograd.Function):
     """softmax(q k^T / sqrt(hd)) v over [L, heads*hd] operands; the core of nn.MultiheadAttention in the adapter.
     ``kv`` None: separate k, v.  Otherwise k | v are the two halves of ``kv`` [Lk, 2 E'] (the output of one fused
     projection GEMM), read in place through row strides, and the gradient comes back as one [Lk, 2 E'] tensor: no split /
-    concat copies on either side."""
+    concat copies on either side.  Returns (o, lse [Lq, heads]); lse is not differentiable (``cross_attn_probs`` input)."""
 
     @staticmethod
     def forward(ctx, q, k, v, kv, heads):
@@ -564,10 +582,12 @@ class CrossAttnFn(torch.autograd.Function):
         o, lse = cross_attn_fwd(q, k, v, heads)
         ctx.save_for_backward(q, k, v, o, lse)
         ctx.heads, ctx.packed = heads, kv is not None
-        return o
+        ctx.mark_non_differentiable(lse)
+        ctx.set_materialize_grads(False)   # no zero-filled gradient for lse in every backward
+        return o, lse
 
     @staticmethod
-    def backward(ctx, d_o):
+    def backward(ctx, d_o, _dlse):
         q, k, v, o, lse = ctx.saved_tensors
         dq, dk, dv = cross_attn_bwd(q, k, v, o, d_o.contiguous().to(q.dtype), lse, ctx.heads, packed_kv=ctx.packed)
         if ctx.packed:
@@ -576,13 +596,15 @@ class CrossAttnFn(torch.autograd.Function):
         return dq.to(q.dtype), dk.to(k.dtype), dv.to(v.dtype), None, None
 
 
-def cross_attention(q, k, v, heads: int):
-    return CrossAttnFn.apply(q, k, v, None, heads)
+def cross_attention(q, k, v, heads: int, return_lse: bool = False):
+    o, lse = CrossAttnFn.apply(q, k, v, None, heads)
+    return (o, lse) if return_lse else o
 
 
-def cross_attention_kv(q, kv, heads: int):
+def cross_attention_kv(q, kv, heads: int, return_lse: bool = False):
     """``cross_attention`` with k | v given as one [Lk, 2 E'] tensor."""
-    return CrossAttnFn.apply(q, None, None, kv, heads)
+    o, lse = CrossAttnFn.apply(q, None, None, kv, heads)
+    return (o, lse) if return_lse else o
 
 
 def gated_residual_fwd(a, b, g32, out=None):

@@ -295,6 +295,8 @@ class GraphedStep:
                 v.copy_(packed_example[k], non_blocking=True)
         self._copy_stream, self._staging, self._staged_for = None, None, None
         self._warmup, self._pool = warmup, pool
+        from .adapter_modules import MultiheadAttention
+        self._attn_modules = [(n, m) for n, m in model.named_modules() if isinstance(m, MultiheadAttention)]
         self._capture()
 
     def _capture_signature(self):
@@ -308,7 +310,18 @@ class GraphedStep:
         (``ops.FrozenLayerWeights``): a ``load_state_dict`` / in-place edit after capture changes it."""
         return tuple((p.data_ptr(), p._version) for p in self.model.parameters() if not p.requires_grad)
 
+    def _check_no_hooks(self):
+        """A forward hook on an attention module runs on the host: it would run once while the graph is captured and
+        never on a replay."""
+        from .adapter_modules import hooked_attention
+        hooked = hooked_attention(self._attn_modules)
+        if hooked:
+            raise RuntimeError("cannot capture or replay a CUDA graph of a model with forward hooks on "
+                               f"{', '.join(hooked)}: remove them (handle.remove()) or run the step eagerly "
+                               "(train_step.forward_backward)")
+
     def _capture(self):
+        self._check_no_hooks()
         model, projector, flat, warmup = self.model, self.projector, self.flat, self._warmup
         slide = unpack_slide(self.static, self.sizes)
         side = torch.cuda.Stream()
@@ -394,6 +407,7 @@ class GraphedStep:
         """``reduce``: all-reduce the flat gradients over the data-parallel ranks after the replay (one slide per rank and
         step).  ``GraphCache`` passes False: ranks step through different numbers of slides and exchange the accumulated
         gradients once."""
+        self._check_no_hooks()
         if self._capture_signature() != self._signature:
             # the graph holds pointers to bf16 copies derived from the old frozen weights, or was captured with the
             # other setting of the deterministic switch: capture again
