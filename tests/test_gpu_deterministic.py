@@ -21,6 +21,7 @@ if ROOT not in sys.path:
 
 from modaltune_b200 import config, ops  # noqa: E402
 from modaltune_b200.slide_encoder import DILATED_RATIO, optimal_segment_lengths  # noqa: E402
+from tests.dilated_ref64 import bwd_ref64  # noqa: E402
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
@@ -92,44 +93,6 @@ def _dilated_inputs(N, sl=None, ratios=None):
     return geom, qkv, dattn, lse, delta
 
 
-def _dilated_bwd_ref64(geom, qkv, dattn, lse, delta):
-    """float64 backward of the dilated core from the kernel's own operands: per (branch, segment, head) the sparse slots
-    p = lo + off + j r (j < m; p >= N are the reference's zero keys), P = exp(S - lse), dS = P (dO V^T - delta_b)."""
-    N, H, D = geom.n_tokens, 16, 48
-    sc = D ** -0.5
-    x = qkv[:N].double()
-    do = dattn[:N].double()
-    out = torch.zeros(N, 3 * 768, dtype=torch.float64, device=qkv.device)
-    lse64 = lse.double()
-    boff = 0
-    for sl, r in zip(geom.segment_lengths, geom.ratios):
-        g = min(sl, N)
-        m = -(-g // r)
-        hpb = H // r
-        dlt = delta[boff: boff + N * hpb].double().view(N, hpb)
-        boff += N * hpb
-        for s in range(-(-N // g)):
-            lo = s * g
-            for h in range(H):
-                off = (h * r) // H
-                pos = lo + off + r * torch.arange(m, device=qkv.device)
-                real = pos < N
-                pr = pos[real]
-                if pr.numel() == 0:
-                    continue
-                cq, ck, cv = slice(h * D, h * D + D), slice(768 + h * D, 768 + h * D + D), slice(1536 + h * D, 1536 + h * D + D)
-                k = torch.zeros(m, D, dtype=torch.float64, device=qkv.device)
-                v = torch.zeros(m, D, dtype=torch.float64, device=qkv.device)
-                k[real], v[real] = x[pr, ck], x[pr, cv]
-                q, dO = x[pr, cq], do[pr, cq]
-                P = torch.exp(q @ k.T * sc - lse64[pr, h][:, None])
-                dS = P * (dO @ v.T - dlt[pr, h - off * hpb][:, None])
-                out[pr, cq] += dS @ k * sc
-                out[pr, ck] += (dS.T @ q * sc)[real]
-                out[pr, cv] += (P.T @ dO)[real]
-    return out
-
-
 @pytest.mark.parametrize("N", SIZES)
 def test_dilated_bwd_impl4_vs_float64_and_repeat(N):
     geom, qkv, dattn, lse, delta = _dilated_inputs(N)
@@ -138,9 +101,11 @@ def test_dilated_bwd_impl4_vs_float64_and_repeat(N):
     torch.cuda.synchronize()
     assert torch.isfinite(a).all()
     assert_bitwise_equal(a, b, f"impl 4 repeat N={N}")
-    ref = _dilated_bwd_ref64(geom, qkv, dattn, lse, delta)
+    ref, tabs = bwd_ref64(geom, qkv, dattn, lse, delta)
     for name, cols in (("dq", slice(0, 768)), ("dk", slice(768, 1536)), ("dv", slice(1536, 2304))):
         got, want = a[:, cols].double(), ref[:, cols]
+        # per element: the bound of the tcgen05 backward (tests/test_gpu_dilated_sm100_ref64.py)
+        within_abs_terms(got, want, tabs[:, cols], 2.0 ** -7, name)
         # the bars of the tcgen05 backward tests of impls 1 / 2 (tests/test_gpu_kernels.py)
         e = float((got - want).abs().max() / want.abs().max())
         assert e < 3e-2, (name, e)
