@@ -132,7 +132,8 @@ int mt_gelu_ln_bwd(const void* dy, int dy_dtype, const void* h, int h_dtype, con
  * C[M, N] = A[M, K] . W[N, K]^T with bf16 operands (row strides lda / ldw in elements), fp32 accumulation in TMEM;
  * N must be a multiple of 256 and K of 64.  What happens to the accumulator is the epilogue `mode`:
  *   MT_EPI_PLAIN        out = acc [+ bias] [+ residual]                       (f32 and / or bf16 output)
- *   MT_EPI_GELU_STATS   h = acc + bias (out_f32, optional);  out_bf16 = u = gelu_erf(h);  out_aux_bf16 = gelu'(h) (optional);
+ *   MT_EPI_GELU_STATS   h = acc + bias (out_f32, optional);  out_bf16 = u = gelu_erf(h);  out_aux_bf16 = gelu'(h) (optional;
+ *                       with neither h nor gelu'(h) the call is the forward-only fc1: same u and stats, no backward state);
  *                       stats[row][slab] = (sum u, sum u^2) of the
  *                       ROUNDED u over each 128-column slab (`stats` is [M, N / 128, 2], every entry written once, no
  *                       atomics: deterministic): fc1 + GELU + the statistics of ffn_layernorm
@@ -163,8 +164,8 @@ typedef struct {
   float* out_f32;           /* [M, N] or NULL, row stride ld_out_f32 (0 = N)                                     */
   void* out_bf16;           /* [M, N] or NULL, row stride ld_out_bf16 (0 = N)                                    */
   int64_t ld_out_f32, ld_out_bf16, ld_residual;
-  void* out_aux_bf16;       /* MT_EPI_GELU_STATS: [M, N] gelu'(h) in bf16 or NULL (then out_f32 = h is required): with  */
-                            /*   it the backward needs neither h nor a second erf / exp per element                    */
+  void* out_aux_bf16;       /* MT_EPI_GELU_STATS: [M, N] gelu'(h) in bf16 or NULL: with it the backward needs neither   */
+                            /*   h nor a second erf / exp per element; a backward needs out_f32 (h) or this            */
   const void* in_u_bf16;    /* MT_EPI_GELU_LN_BWD: gelu(h) and gelu'(h) [M, N] bf16 as written by MT_EPI_GELU_STATS,   */
   const void* in_g_bf16;    /*   used instead of h (`residual` NULL)                                                   */
 } mt_linear_epilogue;
@@ -200,6 +201,13 @@ int mt_ffn_bwd_prep(const float* dy, const float* y, const float* x1, const floa
  * kernels trap: the failure surfaces as a CUDA error on the stream, never as silently unwritten outputs. */
 int mt_dilated_attn_fwd(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc, int dtype,
                         void* o_br, float* lse_br, int impl, void* stream);
+/* mt_dilated_attn_fwd over `batch` sequences of the same geometry in one launch (forward only: evaluation, embedding
+ * extraction).  qkv [batch * n_alloc, 3*E]: sequence b occupies rows [b * n_alloc, b * n_alloc + n_tokens) and its rows
+ * from n_tokens on are zero (no other padding between sequences); o_br / lse_br hold `batch` consecutive copies of the
+ * compact per-branch layout above.  Every sequence gets bitwise what mt_dilated_attn_fwd gives it alone (that call is
+ * batch = 1).  impl 0 (SIMT) and 3 (48-key tcgen05 tiles) take any batch in [1, 65535]; impl 1 only batch = 1. */
+int mt_dilated_attn_fwd_batch(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
+                              int batch, int dtype, void* o_br, float* lse_br, int impl, void* stream);
 
 /* ---- A5 (+ inner_attn_ln of A2): LSE merge of the branches fused with LayerNorm -----------------------------------
  * replaces: DilatedAttention.scattering (dilated_attention.py:113-144) + inner_attn_ln (:257-258).

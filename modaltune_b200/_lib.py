@@ -71,6 +71,7 @@ SIGNATURES = {
     "mt_linear_sm100": (c_int, [_P, _I64, _P, _I64, _I64, _I64, _I64, POINTER(LinearEpilogue), _P]),
     "mt_ffn_bwd_prep": (c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I64, _I64, _I64, _P]),
     "mt_dilated_attn_fwd": (c_int, [_G, _P, _I64, _I64, c_int, _P, _P, c_int, _P]),
+    "mt_dilated_attn_fwd_batch": (c_int, [_G, _P, _I64, _I64, c_int, c_int, _P, _P, c_int, _P]),
     "mt_dilated_merge_ln_fwd": (c_int, [_G, _P, _P, c_int, _P, _P, _P, _P, c_float, _P, _P, _P, _P]),
     "mt_dilated_merge_ln_bwd": (c_int, [_G, _P, c_int, _P, _P, _P, _P, _P, c_int, _P, _P, _P]),
     "mt_dilated_attn_bwd": (c_int, [_G, _P, _I64, _I64, _P, _P, _P, c_int, _P, c_int, _P]),

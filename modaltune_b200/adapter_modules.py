@@ -409,10 +409,26 @@ class InteractionBlockWithCls_LongNetViT(InteractionBlockWithCls):
     def forward_full(self, xfull, c, blocks, incremental_state, layer_configs, query_pos=None):
         """``forward`` on the [1, N, 768] buffer that keeps cls at row 0: the reference's ``cat((cls, x))`` and
         ``x[:, :1], x[:, 1:]`` (:492-505) and their backward copies disappear; same arithmetic."""
-        xfull = self.injector.forward_full(xfull, c, query_pos)
+        xfull = self.inject(xfull, c, query_pos)
+        xfull = self.run_layers(xfull, blocks, incremental_state, layer_configs)
+        return xfull, self.extract(xfull, c, query_pos)
+
+    def inject(self, xfull, c, query_pos=None):
+        """The Injector part of ``forward_full``: the modal tokens ``c`` into the tile rows of [1, N, 768] ``xfull``."""
+        return self.injector.forward_full(xfull, c, query_pos)
+
+    @staticmethod
+    def run_layers(xfull, blocks, incremental_state, layer_configs):
+        """The frozen LongNet layers of ``forward_full`` on [B, N, 768] ``xfull`` (B > 1: the task passes of a slide in
+        lockstep, ``LongNetGeneAdapter.forward_tasks``)."""
         for idx, blk in enumerate(blocks):
             xfull, _ = blk(xfull, incremental_state=(incremental_state[idx] if incremental_state is not None else None),
                            **layer_configs)
+        return xfull
+
+    def extract(self, xfull, c, query_pos=None):
+        """The Extractor part of ``forward_full``: the slide tokens of [1, N, 768] ``xfull`` into the modal tokens ``c``;
+        returns the new ``c``."""
         exts = [self.extractor, *(self.extra_extractors or ())]
         if (self.extra_extractors is not None and config.shared_extractor_kv()
                 and not any(_hooked(e.attn.multihead_attn) for e in exts)):
@@ -423,9 +439,9 @@ class InteractionBlockWithCls_LongNetViT(InteractionBlockWithCls):
             kv_all = ops.shared_kv_project(_rows(xfull), torch.cat([w for w, _ in wb], 0), torch.cat([b for _, b in wb], 0), 1)
             for e, kv in zip(exts, torch.split(kv_all, kv_all.shape[1] // len(exts), dim=1)):
                 c = e.forward_full(c, xfull, query_pos, kv=kv)
-            return xfull, c
+            return c
         c = self.extractor.forward_full(c, xfull, query_pos)
         if self.extra_extractors is not None:
             for extractor in self.extra_extractors:
                 c = extractor.forward_full(c, xfull, query_pos)
-        return xfull, c
+        return c

@@ -58,10 +58,15 @@ __device__ __forceinline__ void load_tile(float* dst, const T* __restrict__ base
   }
 }
 
+// blockIdx.y = sequence of a batch: qkv, o_br and lse_br advance by seq_qkv / seq_o / seq_lse elements per sequence
 template <typename T>
 __global__ void __launch_bounds__(256) dilated_fwd_simt_kernel(const SimtParams P, const T* __restrict__ qkv,
-                                                               T* __restrict__ o_br, float* __restrict__ lse_br) {
+                                                               T* __restrict__ o_br, float* __restrict__ lse_br,
+                                                               int64_t seq_qkv, int64_t seq_o, int64_t seq_lse) {
   extern __shared__ float smem[];
+  qkv += blockIdx.y * seq_qkv;
+  o_br += blockIdx.y * seq_o;
+  lse_br += blockIdx.y * seq_lse;
   float* Qs = smem;
   float* Ks = Qs + BM * LDQ;
   float* Vs = Ks + BM * LDQ;
@@ -509,19 +514,29 @@ static int make_simt_params(const mt_dilated_geometry* geom, int64_t qkv_ld, Sim
   return 0;
 }
 
-int dilated_attn_fwd_simt(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int dtype, void* o_br,
-                          float* lse_br, cudaStream_t st) {
+int dilated_attn_fwd_simt(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc, int batch,
+                          int dtype, void* o_br, float* lse_br, cudaStream_t st) {
   SimtParams P;
   int rc = make_simt_params(geom, qkv_ld, &P);
   if (rc) return rc;
-  const int total = P.item_prefix[P.geo.nb];
+  MT_REQUIRE(batch >= 1 && batch <= 65535, "dilated_attn_fwd: batch must be in [1, 65535] (got %d)", batch);
+  MT_REQUIRE(batch == 1 || n_alloc >= P.geo.N, "dilated_attn_fwd: n_alloc < n_tokens");
+  int64_t seq_o = 0, seq_lse = 0;
+  for (int b = 0; b < P.geo.nb; ++b) {
+    seq_o += (int64_t)P.geo.N * P.geo.b[b].hpb * D;
+    seq_lse += (int64_t)P.geo.N * P.geo.b[b].hpb;
+  }
+  const int64_t seq_qkv = n_alloc * qkv_ld;
+  const dim3 grid(P.item_prefix[P.geo.nb], batch);
   const size_t smem = (size_t)(3 * BM * LDQ + BM * LDP) * sizeof(float);
   if (dtype == MT_F32) {
     MT_CUDA(cudaFuncSetAttribute(dilated_fwd_simt_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dilated_fwd_simt_kernel<float><<<total, 256, smem, st>>>(P, (const float*)qkv, (float*)o_br, lse_br);
+    dilated_fwd_simt_kernel<float><<<grid, 256, smem, st>>>(P, (const float*)qkv, (float*)o_br, lse_br, seq_qkv, seq_o,
+                                                            seq_lse);
   } else {
     MT_CUDA(cudaFuncSetAttribute(dilated_fwd_simt_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    dilated_fwd_simt_kernel<__nv_bfloat16><<<total, 256, smem, st>>>(P, (const __nv_bfloat16*)qkv, (__nv_bfloat16*)o_br, lse_br);
+    dilated_fwd_simt_kernel<__nv_bfloat16><<<grid, 256, smem, st>>>(P, (const __nv_bfloat16*)qkv, (__nv_bfloat16*)o_br,
+                                                                    lse_br, seq_qkv, seq_o, seq_lse);
   }
   return check_launch("dilated_fwd_simt_kernel");
 }
@@ -544,7 +559,7 @@ int dilated_attn_bwd_simt(const mt_dilated_geometry* geom, const void* qkv, int6
 }
 
 // implemented in dilated_sm100.cu
-int dilated_attn_fwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
+int dilated_attn_fwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc, int batch,
                            void* o_br, float* lse_br, int impl, cudaStream_t st);
 int dilated_attn_bwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
                            const void* dattn, const float* lse, const float* delta_br, float* dqkv, int impl,
@@ -554,13 +569,20 @@ int dilated_attn_bwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int
 
 using namespace mt;
 
-extern "C" int mt_dilated_attn_fwd(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
-                                   int dtype, void* o_br, float* lse_br, int impl, void* stream) {
+extern "C" int mt_dilated_attn_fwd_batch(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld,
+                                         int64_t n_alloc, int batch, int dtype, void* o_br, float* lse_br, int impl,
+                                         void* stream) {
   MT_REQUIRE(dtype == MT_F32 || dtype == MT_BF16, "dilated_attn_fwd: bad dtype %d", dtype);
   MT_REQUIRE(qkv_ld % 8 == 0, "dilated_attn_fwd: qkv row stride must be a multiple of 8 elements");
-  if (impl == 0) return dilated_attn_fwd_simt(geom, qkv, qkv_ld, dtype, o_br, lse_br, (cudaStream_t)stream);
+  if (impl == 0)
+    return dilated_attn_fwd_simt(geom, qkv, qkv_ld, n_alloc, batch, dtype, o_br, lse_br, (cudaStream_t)stream);
   MT_REQUIRE(dtype == MT_BF16, "dilated_attn_fwd: the tcgen05 path computes in bf16");
-  return dilated_attn_fwd_sm100(geom, qkv, qkv_ld, n_alloc, o_br, lse_br, impl, (cudaStream_t)stream);
+  return dilated_attn_fwd_sm100(geom, qkv, qkv_ld, n_alloc, batch, o_br, lse_br, impl, (cudaStream_t)stream);
+}
+
+extern "C" int mt_dilated_attn_fwd(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
+                                   int dtype, void* o_br, float* lse_br, int impl, void* stream) {
+  return mt_dilated_attn_fwd_batch(geom, qkv, qkv_ld, n_alloc, 1, dtype, o_br, lse_br, impl, stream);
 }
 
 extern "C" int mt_dilated_attn_bwd(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,

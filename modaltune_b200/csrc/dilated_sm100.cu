@@ -95,6 +95,7 @@ struct Sm100Params {
   int tiles[MT_MAX_BRANCHES];            // 128-slot tiles per (segment, head), indexed by branch
   float scale_log2;                      // head_dim^-0.5 * log2(e)
   float scale;
+  int64_t o_seq, lse_seq;                // elements of o_br / lse_br per sequence (batched forward: blockIdx.y)
 };
 
 // smem carve-up (dynamic, base must be 1024-byte aligned)
@@ -510,14 +511,16 @@ dilated_fwd_sm100_k48_kernel(const __grid_constant__ TensorMaps maps, const __gr
     if (lane == 0) {
       const void* map = &maps.m[b];
       const void* kmap = &kv_maps.m[b];    // the same view with a 48-slot box
+      const int seq = blockIdx.y;          // the 4th map dimension: the zero fill stays inside this sequence
       mbar_expect_tx(bar_q_full, TILE_BYTES);
-      tma_load_3d(sbase + Fwd48Smem::Q, map, bar_q_full, h * DH, off, jseg + q0);
+      tma_load_4d(sbase + Fwd48Smem::Q, map, bar_q_full, h * DH, off, jseg + q0, seq);
       for (int j = 0; j < n_kv; ++j) {
         const int st = j % KS, use = j / KS;
         mbar_wait(bar_kv_empty + 8 * st, (use & 1) ^ 1);
         mbar_expect_tx(bar_kv_full + 8 * st, 2 * KT_BYTES);
-        tma_load_3d(sbase + Fwd48Smem::K + st * KT_BYTES, kmap, bar_kv_full + 8 * st, E + h * DH, off, jseg + j * KT);
-        tma_load_3d(sbase + Fwd48Smem::V + st * KT_BYTES, kmap, bar_kv_full + 8 * st, 2 * E + h * DH, off, jseg + j * KT);
+        tma_load_4d(sbase + Fwd48Smem::K + st * KT_BYTES, kmap, bar_kv_full + 8 * st, E + h * DH, off, jseg + j * KT, seq);
+        tma_load_4d(sbase + Fwd48Smem::V + st * KT_BYTES, kmap, bar_kv_full + 8 * st, 2 * E + h * DH, off, jseg + j * KT,
+                    seq);
       }
     }
   } else if (warp == W_MMA) {
@@ -714,7 +717,8 @@ dilated_fwd_sm100_k48_kernel(const __grid_constant__ TensorMaps maps, const __gr
     if (slot < bg.m && pos < seg_end) {
       const float inv = 1.f / l_run;
       const int slot_h = h - off * bg.hpb;
-      __nv_bfloat16* dst = o_br + bg.o_off + ((int64_t)pos * bg.hpb + slot_h) * DH + half * OC;
+      const int64_t seq = blockIdx.y;
+      __nv_bfloat16* dst = o_br + seq * P.o_seq + bg.o_off + ((int64_t)pos * bg.hpb + slot_h) * DH + half * OC;
 #pragma unroll
       for (int c = 0; c < OC / 8; ++c) {
         uint4 u;
@@ -724,7 +728,7 @@ dilated_fwd_sm100_k48_kernel(const __grid_constant__ TensorMaps maps, const __gr
         u.w = pack_bf16(o_acc[c * 8 + 6] * inv, o_acc[c * 8 + 7] * inv);
         *reinterpret_cast<uint4*>(dst + c * 8) = u;
       }
-      if (half == 0) lse_br[bg.lse_off + (int64_t)pos * bg.hpb + slot_h] = m_used * P.scale + logf(l_run);
+      if (half == 0) lse_br[seq * P.lse_seq + bg.lse_off + (int64_t)pos * bg.hpb + slot_h] = m_used * P.scale + logf(l_run);
     }
   }
   // ---- teardown ------------------------------------------------------------------------------------------------------
@@ -754,18 +758,22 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// 3-D view of a row-major [n_alloc, ld] bf16 matrix for dilation r: (column, residue o, slot j) -> row j*r + o
-static int encode_branch_map(CUtensorMap* map, const void* base, int64_t ld, int64_t n_alloc, int r, int box_rows = BT) {
+// 3-D view of a row-major [n_alloc, ld] bf16 matrix for dilation r: (column, residue o, slot j) -> row j*r + o.
+// batch > 0: 4-D view of `batch` such matrices stacked [batch * n_alloc, ld], (column, residue o, slot j, sequence b) ->
+// row b * n_alloc + j*r + o; slots past n_alloc / r are zero-filled per sequence, never read from the next one.
+static int encode_branch_map(CUtensorMap* map, const void* base, int64_t ld, int64_t n_alloc, int r, int box_rows = BT,
+                             int batch = 0) {
   EncodeTiledFn fn = get_encode_fn();
   if (fn == nullptr) {
     set_error("cuTensorMapEncodeTiled is not available from the driver");
     return MT_E_UNSUPPORTED;
   }
-  cuuint64_t dims[3] = {(cuuint64_t)ld, (cuuint64_t)r, (cuuint64_t)(n_alloc / r)};
-  cuuint64_t strides[2] = {(cuuint64_t)ld * 2, (cuuint64_t)ld * 2 * (cuuint64_t)r};
-  cuuint32_t box[3] = {64, 1, (cuuint32_t)box_rows};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult rc = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
+  const cuuint32_t rank = batch > 0 ? 4 : 3;
+  cuuint64_t dims[4] = {(cuuint64_t)ld, (cuuint64_t)r, (cuuint64_t)(n_alloc / r), (cuuint64_t)batch};
+  cuuint64_t strides[3] = {(cuuint64_t)ld * 2, (cuuint64_t)ld * 2 * (cuuint64_t)r, (cuuint64_t)ld * 2 * (cuuint64_t)n_alloc};
+  cuuint32_t box[4] = {64, 1, (cuuint32_t)box_rows, 1};
+  cuuint32_t estr[4] = {1, 1, 1, 1};
+  CUresult rc = fn(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, rank, const_cast<void*>(base), dims, strides, box, estr,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (rc != CUDA_SUCCESS) {
@@ -829,6 +837,11 @@ static int make_sm100_params(const mt_dilated_geometry* geom, Sm100Params* P) {
   P->item_prefix[nb] = total;
   P->scale = 1.0f / sqrtf((float)DH);
   P->scale_log2 = P->scale * 1.4426950408889634f;
+  P->o_seq = P->lse_seq = 0;
+  for (int b = 0; b < nb; ++b) {
+    P->o_seq += (int64_t)P->geo.N * P->geo.b[b].hpb * DH;
+    P->lse_seq += (int64_t)P->geo.N * P->geo.b[b].hpb;
+  }
   return 0;
 }
 
@@ -847,24 +860,26 @@ static int* next_work_counter() {
   return ring[dev] + 2 * (seq++ % 256);
 }
 
-int dilated_attn_fwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc,
+int dilated_attn_fwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int64_t qkv_ld, int64_t n_alloc, int batch,
                            void* o_br, float* lse_br, int impl, cudaStream_t st) {
   Sm100Params P;
   int rc = make_sm100_params(geom, &P);
   if (rc) return rc;
   MT_REQUIRE(n_alloc >= P.geo.N && n_alloc % 128 == 0, "dilated_attn_fwd: n_alloc must be a multiple of 128 >= n_tokens");
   MT_REQUIRE(qkv_ld % 8 == 0 && ((uintptr_t)qkv & 15) == 0, "dilated_attn_fwd: qkv must be 16-byte aligned");
+  MT_REQUIRE(batch >= 1 && batch <= 65535, "dilated_attn_fwd: batch must be in [1, 65535] (got %d)", batch);
+  MT_REQUIRE(batch == 1 || impl == 3, "dilated_attn_fwd: batch > 1 runs on impl 0 (SIMT) or 3 (48-key tiles) only");
   TensorMaps maps;
   memset(&maps, 0, sizeof(maps));
   for (int b = 0; b < P.geo.nb; ++b) {
-    rc = encode_branch_map(&maps.m[b], qkv, qkv_ld, n_alloc, P.geo.b[b].r);
+    rc = encode_branch_map(&maps.m[b], qkv, qkv_ld, n_alloc, P.geo.b[b].r, BT, impl == 3 ? batch : 0);
     if (rc) return rc;
   }
-  if (impl == 3) {   // 48-key score tiles, four CTAs per SM
+  if (impl == 3) {   // 48-key score tiles, four CTAs per SM; blockIdx.y = sequence
     TensorMaps kv_maps;
     memset(&kv_maps, 0, sizeof(kv_maps));
     for (int b = 0; b < P.geo.nb; ++b) {
-      rc = encode_branch_map(&kv_maps.m[b], qkv, qkv_ld, n_alloc, P.geo.b[b].r, KT);
+      rc = encode_branch_map(&kv_maps.m[b], qkv, qkv_ld, n_alloc, P.geo.b[b].r, KT, batch);
       if (rc) return rc;
     }
     static bool attr_set = false;
@@ -872,7 +887,7 @@ int dilated_attn_fwd_sm100(const mt_dilated_geometry* geom, const void* qkv, int
       MT_CUDA(cudaFuncSetAttribute(dilated_fwd_sm100_k48_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, Fwd48Smem::TOTAL));
       attr_set = true;
     }
-    dilated_fwd_sm100_k48_kernel<<<P.item_prefix[P.geo.nb], FWD_THREADS, Fwd48Smem::TOTAL, st>>>(
+    dilated_fwd_sm100_k48_kernel<<<dim3(P.item_prefix[P.geo.nb], batch), FWD_THREADS, Fwd48Smem::TOTAL, st>>>(
         maps, kv_maps, P, (__nv_bfloat16*)o_br, lse_br);
     return check_launch("dilated_fwd_sm100_k48_kernel");
   }

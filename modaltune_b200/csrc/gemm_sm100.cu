@@ -500,8 +500,7 @@ extern "C" int mt_linear_sm100(const void* a, int64_t lda, const void* w, int64_
                  ep->mode == MT_EPI_GELU_LN_BWD, "linear_sm100: bad epilogue mode %d", ep->mode);
   MT_REQUIRE(ep->out_f32 != nullptr || ep->out_bf16 != nullptr, "linear_sm100: no output");
   if (ep->mode == MT_EPI_GELU_STATS)
-    MT_REQUIRE(ep->bias && ep->out_bf16 && ep->stats && (ep->out_f32 || ep->out_aux_bf16),
-               "linear_sm100: GELU epilogue needs bias, the bf16 output, stats and h (out_f32) or gelu' (out_aux_bf16)");
+    MT_REQUIRE(ep->bias && ep->out_bf16 && ep->stats, "linear_sm100: GELU epilogue needs bias, the bf16 output and stats");
   MT_REQUIRE(ep->out_aux_bf16 == nullptr || ep->mode == MT_EPI_GELU_STATS, "linear_sm100: out_aux_bf16 belongs to the GELU epilogue");
   if (ep->mode == MT_EPI_LN_RESIDUAL)
     MT_REQUIRE(ep->col_c1 && ep->col_c2 && ep->stats && ep->ln_cols > 0, "linear_sm100: LN-fold epilogue needs c1, c2, stats, ln_cols");

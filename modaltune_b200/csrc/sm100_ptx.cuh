@@ -71,6 +71,15 @@ __device__ __forceinline__ void tma_load_3d(uint32_t dst, const void* desc, uint
       : "memory");
 }
 
+__device__ __forceinline__ void tma_load_4d(uint32_t dst, const void* desc, uint32_t bar, int c0, int c1, int c2,
+                                            int c3) {
+  asm volatile(
+      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+      :
+      : "r"(dst), "l"(reinterpret_cast<uint64_t>(desc)), "r"(bar), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
+      : "memory");
+}
+
 __device__ __forceinline__ void tma_load_2d(uint32_t dst, const void* desc, uint32_t bar, int c0, int c1) {
   asm volatile(
       "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"

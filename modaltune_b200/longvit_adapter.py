@@ -14,9 +14,9 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import config
+from . import config, ops
 from .adapter_modules import (CrossAttentionLayer, Identity_mod, InteractionBlockWithCls_LongNetViT,
-                              SelfAttentionLayer, recording_outputs)
+                              MultiheadAttention, SelfAttentionLayer, hooked_attention, recording_outputs)
 from .gene_encoder import GeneEncoder_Group
 from .slide_encoder import LongNetViT
 
@@ -151,10 +151,16 @@ class LongNetGeneAdapter(LongNetViT):
         ``split_grads``: every pass reads the trainable parameters through its OWN leaf aliases (same storage, listed in
         ``self._pass_aliases`` for the caller, ``train_step.forward_backward``).  The autograd engine then delivers one
         gradient per (parameter, pass) instead of summing the passes' contributions with two tiny add kernels per
-        parameter (~700 launches per step); the caller sums them with two multi-tensor adds."""
+        parameter (~700 launches per step); the caller sums them with two multi-tensor adds.
+
+        Forward only (``_lockstep``: no autograd, eval mode, bf16 mode with the tcgen05 GEMMs, no hooked attention module)
+        the passes run in lockstep: each block's frozen layers run ONCE on the [T, N, 768] stack of the passes' residual
+        streams (``_forward_lockstep``), the same arithmetic as T separate passes, bit for bit."""
         emb = self.embed(x, coords)
         gene = None if self.training else self.gene_encoder(genes)
         self._pass_aliases = None
+        if self._lockstep(len(task_tokens)):
+            return self._forward_lockstep(emb, gene, clinical, task_tokens)
         if split_grads and config.flag("split_param_grads") and torch.is_grad_enabled() and len(task_tokens) > 1:
             # the gene encoder stays on the shared leaves: in eval mode it runs once for all passes, and in train mode its
             # 1 324 per-pathway gradients are strided slices of stacked tensors, which the multi-tensor add of
@@ -204,6 +210,41 @@ class LongNetGeneAdapter(LongNetViT):
             tns.record_stream(cur)
         return torch.cat(outs, 0)
 
+    def _lockstep(self, n_tasks: int) -> bool:
+        """Run ``n_tasks`` passes in lockstep?  Only when the frozen layers take the stack as one batch
+        (``LongNetEncoderLayer.runs_batched``) and no forward hook on an attention module would see its calls reordered."""
+        if n_tasks < 2 or self.training or torch.is_grad_enabled() or not ops.batched_forward_available():
+            return False
+        mods = self.__dict__.get("_attn_modules")
+        if mods is None:
+            mods = self.__dict__["_attn_modules"] = [(n, m) for n, m in self.named_modules()
+                                                     if isinstance(m, MultiheadAttention)]
+        return not hooked_attention(mods)
+
+    def _forward_lockstep(self, emb, gene_tokens, clinical, task_tokens):
+        """``_adapter_forward`` of every task token at once: per block, each pass's prompt self-attention and Injector on
+        its own [1, N, 768] rows, then the block's frozen layers once on the [T, N, 768] stack (cls at row 0 of every
+        pass), then each pass's Extractor(s).  -> [T, output_dim]."""
+        T = len(task_tokens)
+        x, _, encoder_padding_mask, rel_pos_bias = self.encoder.prepare_forward(src_tokens=None, token_embeddings=emb)
+        layer_configs = {"rel_pos": rel_pos_bias, "encoder_padding_mask": encoder_padding_mask, "attn_mask": None,
+                         "multiway_split_position": None}
+        cs = [self._modal_tokens(gene_tokens, clinical, t) for t in task_tokens]
+        first = self.interaction_indexes[0][0]
+        xs = x.expand(T, -1, -1)
+        if first > 0:
+            xs = InteractionBlockWithCls_LongNetViT.run_layers(xs, self.encoder.layers[0:first], None, layer_configs)
+        for i, layer in enumerate(self.interactions):
+            lo, hi = self.interaction_indexes[i][0], self.interaction_indexes[i][-1]
+            outs = []
+            for k in range(T):
+                cs[k] = self.prompt_selfattention[i](cs[k], self.gene_pe)
+                outs.append(layer.inject(xs[k:k + 1], cs[k], self.gene_pe))
+            xs = layer.run_layers(torch.cat(outs, 0), self.encoder.layers[lo:hi + 1], None, layer_configs)
+            for k in range(T):
+                cs[k] = layer.extract(xs[k:k + 1], cs[k], self.gene_pe)
+        return torch.cat([self._outcome(xs[k:k + 1], cs[k]) for k in range(T)], 0)
+
     def join_pass_streams(self):
         """Make the current stream wait for everything queued on the task-pass streams (call after a backward)."""
         streams = self.__dict__.get("_streams", [])
@@ -249,6 +290,10 @@ class LongNetGeneAdapter(LongNetViT):
             c = self.prompt_selfattention[i](c, self.gene_pe)
             x, c = layer.forward_full(x, c, self.encoder.layers[lo:hi + 1], incremental_state, layer_configs,
                                       self.gene_pe)
+        return self._outcome(x, c)
+
+    def _outcome(self, x, c):
+        """The head of a task pass: [1, N, 768] slide tokens and the modal tokens -> [1, output_dim]."""
         img_outcome = x[:, 1:].mean(dim=1).unsqueeze(0) if self.global_pool else x[:, :1]
         if self.add_prompt_feature:
             k = int(self._HAS_CLINICAL)

@@ -278,6 +278,37 @@ def dilated_attn_fwd(geom: Geometry, qkv: torch.Tensor, impl: int):
     return o_br, lse_br
 
 
+def dilated_attn_fwd_batch(geom: Geometry, qkv: torch.Tensor, impl: int):
+    """qkv [B, n_alloc, 3E] (rows >= N of every sequence zero) -> (o_br [B * o_elems], lse_br [B * lse_elems]): B
+    consecutive copies of the compact per-branch layout, one launch; each equals ``dilated_attn_fwd`` of its sequence."""
+    B, n_alloc, _ = qkv.shape
+    assert n_alloc == geom.n_alloc and qkv.is_contiguous()
+    o_br = torch.empty(B * geom.o_elems, device=qkv.device, dtype=qkv.dtype)
+    lse_br = torch.empty(B * geom.lse_elems, device=qkv.device, dtype=torch.float32)
+    with _timed("dilated_attn_fwd"):
+        rc = _lib.load().mt_dilated_attn_fwd_batch(geom.ref(), _p(qkv), qkv.stride(1), n_alloc, B, _dt(qkv), _p(o_br),
+                                                   _p(lse_br), impl, _stream())
+    _check(rc, "mt_dilated_attn_fwd_batch")
+    return o_br, lse_br
+
+
+def dilated_merge_ln_fwd_batch(geom: Geometry, o_br, lse_br, gamma, beta, batch: int, eps: float = LN_EPS):
+    """``dilated_merge_ln_fwd`` of each sequence of a ``dilated_attn_fwd_batch`` output into ONE stacked y [B * N, E]
+    (one launch per sequence on offset pointers); the merged lse and LayerNorm statistics are not kept."""
+    N, E = geom.n_tokens, geom.heads * geom.head_dim
+    y = torch.empty((batch * N, E), device=o_br.device, dtype=o_br.dtype)
+    lse = torch.empty((N, geom.heads), device=o_br.device, dtype=torch.float32)
+    mean = torch.empty(N, device=o_br.device, dtype=torch.float32)
+    rstd = torch.empty(N, device=o_br.device, dtype=torch.float32)
+    lib = _lib.load()
+    for b in range(batch):
+        rc = lib.mt_dilated_merge_ln_fwd(geom.ref(), _p(o_br[b * geom.o_elems:(b + 1) * geom.o_elems]),
+                                         _p(lse_br[b * geom.lse_elems:(b + 1) * geom.lse_elems]), _dt(o_br), None, _p(lse),
+                                         _p(gamma), _p(beta), eps, _p(y[b * N:(b + 1) * N]), _p(mean), _p(rstd), _stream())
+        _check(rc, "mt_dilated_merge_ln_fwd")
+    return y
+
+
 def dilated_merge_ln_fwd(geom: Geometry, o_br, lse_br, gamma, beta, eps: float = LN_EPS, want_attn: bool = False):
     N, E = geom.n_tokens, geom.heads * geom.head_dim
     y = torch.empty((N, E), device=o_br.device, dtype=o_br.dtype)
@@ -1035,6 +1066,45 @@ def _encoder_layer_backward_sm100(dy: torch.Tensor, saved, W: FrozenLayerWeights
     else:
         dx, _, _ = layernorm_bwd(dh1, x, W.ln1[0], mean1, rstd1, torch.float32, residual=dx1)
     return dx
+
+
+def batched_forward_available() -> bool:
+    """Can ``encoder_layer_forward_batch`` run: bf16 mode with the tcgen05 GEMMs.  Every kernel of that forward computes a
+    row (a work item of the attention) the same way whatever the batch, so a batched layer gives each sequence bitwise what
+    a call of its own gives it.  fp32 mode has no such guarantee (cuBLAS may pick another algorithm for a taller M)."""
+    from . import config
+    return config.mode() == "bf16" and config.gemm_impl() == "sm100"
+
+
+def encoder_layer_forward_batch(x: torch.Tensor, W: FrozenLayerWeights, geom: Geometry, batch: int, impl) -> torch.Tensor:
+    """Forward only: B sequences of N tokens through one frozen layer, x [B * N, 768] fp32 (plainly stacked) -> y of the
+    same shape, bitwise ``_encoder_layer_forward_sm100`` of every sequence.  Only the qkv buffer is padded per sequence
+    ([B, n_alloc, 2304], zero tails: the TMA view of the attention reads them); the attention is one launch; the
+    LayerNorms, out_proj, fc1 and fc2 run once over all B * N rows.  fc1 writes neither h nor gelu'(h) (nothing runs a
+    backward), nothing is saved and no layer hand-over is recorded."""
+    N = geom.n_tokens
+    cdt = torch.bfloat16
+    h1, _, _ = layernorm_fwd(x, W.ln1[0], W.ln1[1], cdt)
+    qkv = torch.empty((batch, geom.n_alloc, 3 * EMBED), device=x.device, dtype=cdt)
+    if geom.n_alloc > N:
+        qkv[:, N:].zero_()
+    for b in range(batch):
+        linear_sm100(h1[b * N:(b + 1) * N], W.w_qkv, bias=W.b_qkv32, want_f32=False, out_bf16=qkv[b, :N])
+    del h1
+    o_br, lse_br = dilated_attn_fwd_batch(geom, qkv, impl[0])
+    del qkv
+    a_ln = dilated_merge_ln_fwd_batch(geom, o_br, lse_br, W.ln_in[0], W.ln_in[1], batch)
+    del o_br, lse_br
+    x1, _ = linear_sm100(a_ln, W.w_o, bias=W.b_o, residual=x)
+    del a_ln
+    h2, _, _ = layernorm_fwd(x1, W.ln2[0], W.ln2[1], cdt)
+    stats = torch.empty((batch * N, W.w_1.shape[0] // 128, 2), device=x.device, dtype=torch.float32)
+    u = torch.empty((batch * N, W.w_1.shape[0]), device=x.device, dtype=cdt)
+    linear_sm100(h2, W.w_1, mode=_lib.MT_EPI_GELU_STATS, bias=W.b_1, want_f32=False, out_bf16=u, stats=stats)
+    del h2
+    y, _ = linear_sm100(u, W.w_2g, mode=_lib.MT_EPI_LN_RESIDUAL, residual=x1, stats=stats, col_c1=W.c1_2, col_c2=W.c2_2,
+                        ln_cols=W.w_2g.shape[1])
+    return y
 
 
 def encoder_layer_forward(x: torch.Tensor, W: FrozenLayerWeights, geom: Geometry, cdt: torch.dtype, impl, rng=None):

@@ -99,6 +99,13 @@ class LongNetEncoderLayer(nn.Module):
         self.ratios = [int(r) for r in ratios]
         self._weights = ops.FrozenLayerWeights()
 
+    def runs_batched(self, x) -> bool:
+        """Does a [B, N, 768] input (B > 1) run as ONE batched forward (``ops.encoder_layer_forward_batch``) instead of B
+        layer calls: when autograd records nothing, in eval mode, in bf16 mode with the tcgen05 GEMMs.  Each sequence then
+        gets bitwise what its own call gives it."""
+        return (x.shape[0] > 1 and not (torch.is_grad_enabled() and x.requires_grad) and not self.training
+                and ops.batched_forward_available())
+
     def forward(self, x, encoder_padding_mask=None, attn_mask=None, rel_pos=None, multiway_split_position=None,
                 incremental_state=None):
         assert attn_mask is None and rel_pos is None and incremental_state is None, \
@@ -117,6 +124,9 @@ class LongNetEncoderLayer(nn.Module):
             rng = ops.train_rng(x.device, self.dropout, self.drop_path_prob, 2 * self.layer_index)
         if B == 1:   # pure views: the backward of x[0] would zero-fill and copy a [1, N, 768] gradient per layer
             return ops.frozen_encoder_layer(x.reshape(N, E).float(), W, geom, cdt, impl, rng).unsqueeze(0), None
+        if self.runs_batched(x):
+            y = ops.encoder_layer_forward_batch(x.reshape(B * N, E).float().contiguous(), W, geom, B, impl)
+            return y.view(B, N, E), None
         outs = [ops.frozen_encoder_layer(x[b].float(), W, geom, cdt, impl, rng) for b in range(B)]
         y = torch.stack(outs, 0)
         return y, None

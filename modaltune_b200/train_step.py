@@ -265,7 +265,27 @@ def unpack_slide(packed: Dict, sizes: Sequence[int]) -> Dict:
     return d
 
 
-class GraphedStep:
+class _CapturedModel:
+    """What a CUDA graph of the model depends on besides its inputs, shared by the captured training step and the captured
+    evaluation forward."""
+
+    def _frozen_signature(self):
+        """Identity + version of every frozen parameter the captured kernels read through derived copies
+        (``ops.FrozenLayerWeights``): a ``load_state_dict`` / in-place edit after capture changes it."""
+        return tuple((p.data_ptr(), p._version) for p in self.model.parameters() if not p.requires_grad)
+
+    def _check_no_hooks(self):
+        """A forward hook on an attention module runs on the host: it would run once while the graph is captured and
+        never on a replay."""
+        from .adapter_modules import hooked_attention
+        hooked = hooked_attention(self._attn_modules)
+        if hooked:
+            raise RuntimeError("cannot capture or replay a CUDA graph of a model with forward hooks on "
+                               f"{', '.join(hooked)}: remove them (handle.remove()) or run eagerly "
+                               "(train_step.forward_backward / multitask_forward)")
+
+
+class GraphedStep(_CapturedModel):
     """forward (3 task passes) + loss + backward + gradient flattening of ONE slide shape captured in a CUDA graph.
 
     A step launches ~5 000 kernels, most of them tiny (gene encoder, modal-token side of the adapter, autograd glue);
@@ -304,21 +324,6 @@ class GraphedStep:
         fast backward must never replay as deterministic, nor the other way round) and the frozen weights."""
         from . import config
         return config.deterministic(), self._frozen_signature()
-
-    def _frozen_signature(self):
-        """Identity + version of every frozen parameter the captured kernels read through derived copies
-        (``ops.FrozenLayerWeights``): a ``load_state_dict`` / in-place edit after capture changes it."""
-        return tuple((p.data_ptr(), p._version) for p in self.model.parameters() if not p.requires_grad)
-
-    def _check_no_hooks(self):
-        """A forward hook on an attention module runs on the host: it would run once while the graph is captured and
-        never on a replay."""
-        from .adapter_modules import hooked_attention
-        hooked = hooked_attention(self._attn_modules)
-        if hooked:
-            raise RuntimeError("cannot capture or replay a CUDA graph of a model with forward hooks on "
-                               f"{', '.join(hooked)}: remove them (handle.remove()) or run the step eagerly "
-                               "(train_step.forward_backward)")
 
     def _capture(self):
         self._check_no_hooks()
@@ -429,27 +434,20 @@ class GraphedStep:
         return self.loss, self.logits
 
 
-class GraphCache:
-    """Captured steps for VARIABLE-length slides (pan-cancer training, BASELINE config 5: 2k-40k tiles per slide).
+class _ShapeCache:
+    """One captured graph per token count: all share ONE memory pool and ONE set of static input buffers sized for
+    ``max_tiles`` (replayed one at a time, outputs consumed before the next replay)."""
 
-    A CUDA graph is shape-specific and the eager step is host-bound (~3 000 launches from Python: twice the graph's
-    time at 10k tiles, worse below), but training visits the same slides every epoch: the cache keeps one captured step
-    per token count.  All steps share ONE memory pool and ONE set of static input buffers sized for ``max_tiles`` --
-    they are replayed one at a time and their outputs (loss, logits, flat gradients) are consumed before the next
-    replay -- so a cached shape costs only its graph object, not its 13-50 GB of activations.  The first visit of a shape
-    captures (about the cost of an eager step); every later visit is one graph launch.  ``hits`` / ``misses`` count."""
-
-    def __init__(self, model, projector, flat: FlatGradAllReduce, sizes: Sequence[int], in_chans: int = 1536,
-                 max_tiles: int = 40960, max_entries: int = 4096):
+    def __init__(self, model, sizes: Sequence[int], in_chans: int, max_tiles: int, max_entries: int):
         from collections import OrderedDict
-        self.model, self.projector, self.flat, self.sizes = model, projector, flat, list(sizes)
+        self.model, self.sizes = model, list(sizes)
         dev = next(model.parameters()).device
         self.pool = torch.cuda.graph_pool_handle()
         self.max_tiles, self.max_entries = max_tiles, max_entries
         self._x = torch.empty((max_tiles, in_chans), device=dev, dtype=torch.float32)
         self._coords = torch.empty((max_tiles, 2), device=dev, dtype=torch.float32)
         self._small: Dict[str, torch.Tensor] = {}
-        self.steps: "OrderedDict[int, GraphedStep]" = OrderedDict()
+        self.steps: "OrderedDict[int, object]" = OrderedDict()
         self.hits = self.misses = 0
 
     def _static_for(self, packed: Dict) -> Dict:
@@ -466,6 +464,22 @@ class GraphCache:
                     self._small[k] = torch.empty(v.shape, device=self._x.device, dtype=v.dtype)
                 out[k] = self._small[k]
         return out
+
+
+class GraphCache(_ShapeCache):
+    """Captured steps for VARIABLE-length slides (pan-cancer training, BASELINE config 5: 2k-40k tiles per slide).
+
+    A CUDA graph is shape-specific and the eager step is host-bound (~3 000 launches from Python: twice the graph's
+    time at 10k tiles, worse below), but training visits the same slides every epoch: the cache keeps one captured step
+    per token count.  All steps share ONE memory pool and ONE set of static input buffers sized for ``max_tiles`` --
+    they are replayed one at a time and their outputs (loss, logits, flat gradients) are consumed before the next
+    replay -- so a cached shape costs only its graph object, not its 13-50 GB of activations.  The first visit of a shape
+    captures (about the cost of an eager step); every later visit is one graph launch.  ``hits`` / ``misses`` count."""
+
+    def __init__(self, model, projector, flat: FlatGradAllReduce, sizes: Sequence[int], in_chans: int = 1536,
+                 max_tiles: int = 40960, max_entries: int = 4096):
+        super().__init__(model, sizes, in_chans, max_tiles, max_entries)
+        self.projector, self.flat = projector, flat
 
     def __call__(self, packed: Dict):
         """One slide step (packed host or device tensors, ``pack_host_slide``): (loss, logits); the gradients of THIS
@@ -486,3 +500,97 @@ class GraphCache:
         self.hits += 1
         self.steps.move_to_end(L)
         return step(packed, reduce=False)
+
+
+# ---------------------------------------------------------------------------------------------------------------------
+# CUDA-graph evaluation forward
+# ---------------------------------------------------------------------------------------------------------------------
+class GraphedForward(_CapturedModel):
+    """``multitask_forward(model, slide, task_ids)`` under ``torch.no_grad()`` of ONE slide shape captured in a CUDA graph:
+    what ``evaluate`` / ``get_features`` / ``deploy_mil`` run per slide (train_modaltune.py), without the host-bound eager
+    launch stream.  In eval mode with bf16 and the tcgen05 GEMMs the task passes run in lockstep inside the graph
+    (``LongNetGeneAdapter.forward_tasks``).  Touches no gradient and no training-step state.
+
+    Re-captures when a frozen weight changes (``load_state_dict``) or the model's train / eval mode or compute mode
+    changes; refuses a model with forward hooks on an attention module (``_check_no_hooks``)."""
+
+    def __init__(self, model, packed_example: Dict, sizes: Sequence[int], task_ids: Sequence[int] = (0, 1, 2),
+                 warmup: int = 1, pool=None, static: Optional[Dict] = None):
+        """``pool`` / ``static``: a memory pool and device input buffers shared with other captured forwards
+        (``GraphedForwardCache``), as for ``GraphedStep``."""
+        self.model, self.sizes, self.task_ids = model, list(sizes), tuple(task_ids)
+        dev = next(model.parameters()).device
+        if static is None:
+            self.static = {k: v.to(dev).clone() for k, v in packed_example.items()}
+        else:
+            self.static = static
+            for k, v in self.static.items():
+                assert v.shape == packed_example[k].shape and v.device == dev
+                v.copy_(packed_example[k], non_blocking=True)
+        self._warmup, self._pool = warmup, pool
+        from .adapter_modules import MultiheadAttention
+        self._attn_modules = [(n, m) for n, m in model.named_modules() if isinstance(m, MultiheadAttention)]
+        self._capture()
+
+    def _capture_signature(self):
+        from . import config
+        return self.model.training, config.mode(), config.gemm_impl(), config.attn_impl("fwd"), self._frozen_signature()
+
+    def _capture(self):
+        self._check_no_hooks()
+        slide = unpack_slide(self.static, self.sizes)
+        side = torch.cuda.Stream()
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side), torch.no_grad():
+            for _ in range(self._warmup):
+                multitask_forward(self.model, slide, self.task_ids)
+        torch.cuda.current_stream().wait_stream(side)
+        torch.cuda.synchronize()
+        self.graph = torch.cuda.CUDAGraph()
+        with torch.no_grad(), torch.cuda.graph(self.graph, pool=self._pool):
+            self.logits = multitask_forward(self.model, slide, self.task_ids)
+        self._signature = self._capture_signature()
+
+    def load(self, packed: Dict):
+        """Copy one packed slide (``pack_host_slide``: pinned host or device tensors of the captured shapes) into the
+        static inputs."""
+        for k, v in self.static.items():
+            v.copy_(packed[k], non_blocking=True)
+
+    def __call__(self, packed: Optional[Dict] = None) -> torch.Tensor:
+        """[len(task_ids), 256] logits of ``packed`` (or of the slide already in the static inputs): the captured buffer,
+        valid until the next call."""
+        self._check_no_hooks()
+        if self._capture_signature() != self._signature:
+            self._capture()
+        if packed is not None:
+            self.load(packed)
+        self.graph.replay()
+        return self.logits
+
+
+class GraphedForwardCache(_ShapeCache):
+    """Captured evaluation forwards (``GraphedForward``) for slides of any tile count, one per token count, in ONE memory
+    pool and ONE set of static inputs sized for ``max_tiles`` (as ``GraphCache`` does for the training step): an evaluation
+    epoch captures each new shape once (about the cost of an eager forward) and replays it on every later visit."""
+
+    def __init__(self, model, sizes: Sequence[int], task_ids: Sequence[int] = (0, 1, 2), in_chans: int = 1536,
+                 max_tiles: int = 40960, max_entries: int = 4096):
+        super().__init__(model, sizes, in_chans, max_tiles, max_entries)
+        self.task_ids = tuple(task_ids)
+
+    def __call__(self, packed: Dict) -> torch.Tensor:
+        """[len(task_ids), 256] logits of one packed slide (``pack_host_slide``), valid until the next call."""
+        L = int(packed["x"].shape[-2])
+        fwd = self.steps.get(L)
+        if fwd is None:
+            self.misses += 1
+            if len(self.steps) >= self.max_entries:
+                self.steps.popitem(last=False)
+            fwd = GraphedForward(self.model, packed, self.sizes, self.task_ids, warmup=1 if not self.steps else 0,
+                                 pool=self.pool, static=self._static_for(packed))
+            self.steps[L] = fwd
+            return fwd()
+        self.hits += 1
+        self.steps.move_to_end(L)
+        return fwd(packed)
